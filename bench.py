@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path on BASELINE.json's metric: RANSAC hyp x corr evals/s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one pass of the whole hot path over one synthetic image pair of
 BASELINE config 2 (10,000 correspondences, 30 % outliers, 1 px noise, 65,536
@@ -21,6 +21,11 @@ N ranks, the (count, index) exchange once through NVLink peer memory -
 sfmb200_estimate_e_mg - and once through an NCCL all-reduce; strong scaling),
 `c4` (4,096 pairs x 4k x 4k, PAIRS sharded over the N ranks; strong scaling) and
 `c5` (full path with 1M triangulated points; the triangulation roofline).
+
+--dump-outputs DIR writes, after the K timed steps, what the last of them left for the caller
+(rank 0's pair: the outputs of sfmb200_run_host, read from the device-path handle) as DIR/<name>.npy
+in float32 (E, P, points) or float64 (the integer outputs, exact), so that two builds can be compared
+output for output: the inputs depend on the arguments only.
 
 --impl reference times the reference's OWN implementation of the path, which is
 CUDA (it has no CPU path): its unmodified sources rebuilt for sm_100a as
@@ -197,6 +202,19 @@ def _timed(torch, dist, world, fn, reps):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         out.append(float(t.item()))
     return out
+
+
+def dump_outputs(out_dir: str, h) -> None:
+    """The arrays sfmb200_run_host returns for pair 0 (E, selected pose P, pose index, inlier count, points) plus the
+    winning hypothesis' index and the inlier mask, as the last whole-path call left them on the handle."""
+    best_idx, best_cnt = h.get_best()
+    ind = h.get_pose_index()
+    arrays = {"E": h.get_E().reshape(h.pairs, 9), "P": h.get_poses()[np.arange(h.pairs), ind].reshape(h.pairs, 16),
+              "pose_index": ind, "inliers": best_cnt, "best_hypothesis": best_idx, "points": h.get_points_host(0)[None],
+              "inlier_mask": h.get_inlier_mask().cpu().numpy()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
 
 
 def run_configs(pkg, torch, dist, rank, world, K, Kinv, args) -> dict:
@@ -450,6 +468,8 @@ def run_ours(args):
     total_ms = timed_region(args.steps)
     wall = time.perf_counter() - wall0
     launches = h.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, h)
     ms_per_step = total_ms / args.steps
     value = world * N_HYP * N_CORR / (ms_per_step * 1e-3)
     # second region, same K steps of the same workload, WITH the per-stage CUDA events (recorded on the
@@ -763,7 +783,12 @@ def main():
     ap.add_argument("--ref-child", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--no-extras", action="store_true",
                     help="headline config-2 regions only (for profiler captures: skips the sustained run's companions c1, c3, c4, c5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (--impl ours only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this project's path: use it with --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -309,3 +309,15 @@ def test_svd_h_facade_surface_host_and_device(tmp_path):
     r = subprocess.run([nvcc, "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", f"-I{inc}", "-c", "-o", str(tmp_path / "svdchk.o"), str(cu)],
                        capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
+
+
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]])
+def test_bench_rejects_arguments_it_cannot_honour(args, tmp_path):
+    """Checked before anything runs: no step count below 1, and --dump-outputs only for this project's path (the
+    reference arm has nothing to dump, and an empty directory must not pass for a comparable run)."""
+    import subprocess
+    import sys
+
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True, timeout=120, cwd=tmp_path)
+    assert r.returncode == 2 and "error" in r.stderr and not r.stdout.strip()
+    assert not (tmp_path / "unused").exists()

@@ -104,12 +104,15 @@ def test_whole_path_is_cuda_graph_capturable(pkg, O):
         h.close()
 
 
-def test_bench_json_contract_reduced_extras():
+def test_bench_json_contract_reduced_extras(tmp_path):
     """bench.py prints ONE JSON line with the contract's keys; the extra configs run at a reduced scale here
-    (SFMB200_BENCH_SCALE shrinks configs 3-5 only: the headline config 2 is always full size)."""
+    (SFMB200_BENCH_SCALE shrinks configs 3-5 only: the headline config 2 is always full size).  --dump-outputs writes
+    the last timed step's outputs, and they agree with what the line reports."""
+    import numpy as np
+
     env = dict(os.environ, SFMB200_BENCH_SCALE="0.01")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "5", "--warmup", "3"], capture_output=True, text=True,
-                       timeout=900, env=env)
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "5", "--warmup", "3", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900, env=env)
     assert r.returncode == 0, r.stderr[-2000:]
     out = [l for l in r.stdout.strip().splitlines() if l.strip()]
     assert len(out) == 1, out[:3]
@@ -127,6 +130,20 @@ def test_bench_json_contract_reduced_extras():
     assert d["c1"]["winner"] == d["c1"]["winner_fixture_fp64"] or abs(d["c1"]["winner"][1] - d["c1"]["winner_fixture_fp64"][1]) <= 3
     assert d["roofline_triangulation"]["frac"] is not None and d["c4"]["pairs"] >= 1
     assert d["sustained"]["wall_s"] >= 1.5 and not set(d["clocks"]["reasons"]) & {"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"}
+    o = {k: np.load(tmp_path / f"{k}.npy") for k in ("E", "P", "pose_index", "inliers", "best_hypothesis", "points", "inlier_mask")}
+    assert all(a.dtype in (np.float32, np.float64) for a in o.values())
+    assert o["E"].shape == (1, 9) and o["P"].shape == (1, 16) and o["points"].shape == (1, 4, 10000) and o["inlier_mask"].shape == (10000,)
+    res = d["result"]
+    assert int(o["inliers"][0]) == int(o["inlier_mask"].sum()) == res["inliers"]
+    assert int(o["best_hypothesis"][0]) == res["best_hypothesis"] and int(o["pose_index"][0]) == res["pose_index"]
+    assert np.all(o["points"][0, 3] == 1)
+    # the same arguments again (the companion configs run after the dump, so they are left out): the same outputs, bit for bit
+    again = tmp_path / "again"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "5", "--warmup", "3", "--no-extras", "--dump-outputs", str(again)],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    for k, a in o.items():
+        assert np.array_equal(np.load(again / f"{k}.npy"), a), k
 
 
 def test_bench_reference_arm_survives_a_dying_reference():
