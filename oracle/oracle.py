@@ -506,6 +506,18 @@ def match_candidates(Pa: np.ndarray, Pb: np.ndarray, tol: float = 1e-3):
     return None
 
 
+def match_candidate_set(Pa: np.ndarray, Pb: np.ndarray, tol: float = 1e-4):
+    """Textbook candidates (compat=False) come from an SVD whose orientation is free, so their order is too: parity
+    means equal as a SET.  Returns a bijection perm with |Pa[i] - Pb[perm[i]]| < tol, or None."""
+    import itertools
+
+    Pa, Pb = np.asarray(Pa, float).reshape(4, 4, 4), np.asarray(Pb, float).reshape(4, 4, 4)
+    for perm in itertools.permutations(range(4)):
+        if all(np.abs(Pa[i] - Pb[perm[i]]).max() < tol for i in range(4)):
+            return perm
+    return None
+
+
 def dlt_rows(x: np.ndarray, M: np.ndarray) -> np.ndarray:
     """compute_linear_triangulation_A (kernels.h:387-431): per point the 4x4
     [x1*I[2]-I[0]; y1*I[2]-I[1]; x2*M[2]-M[0]; y2*M[2]-M[1]] with camera 1 = I4."""
@@ -551,13 +563,19 @@ def choose_pose(x: np.ndarray, P: np.ndarray, compat: bool = True, mask: np.ndar
             if z1 > 0 and z2 > 0:
                 ind = i
         return ind, Pinv
+    return int(np.argmax(cheirality_votes(x, P, mask))), P.copy()
+
+
+def cheirality_votes(x: np.ndarray, P: np.ndarray, mask: np.ndarray | None = None, tri=triangulate) -> list[int]:
+    """Votes of choosePose's correct mode: per candidate, the (masked) points whose triangulation lies in front of both
+    cameras.  tri(x, M) -> (4,n) is the triangulation to use (default: this module's fp64 SVD)."""
     xs = x if mask is None else x[mask]
     votes = []
     for i in range(4):
-        X = triangulate(xs, P[i])
+        X = tri(xs, P[i])
         z2 = (P[i] @ X)[2]
         votes.append(int(((X[2] > 0) & (z2 > 0)).sum()))
-    return int(np.argmax(votes)), P.copy()
+    return votes
 
 
 # --------------------------------------------------------------------------

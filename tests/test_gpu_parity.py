@@ -286,6 +286,40 @@ def test_correct_mode_recovers_ground_truth_pose(pkg, O, torch_cuda):
     h.close()
 
 
+@pytest.mark.parametrize("seed", [5, 61])
+@pytest.mark.parametrize("B", [1, 3])
+@pytest.mark.parametrize("n", [700, 5000])
+def test_vote_mode_poses_against_oracle(pkg, O, torch_cuda, seed, B, n):
+    """SFMB200_OPT_COMPAT = 0 (textbook candidates + inlier vote) and inliers-only triangulation against the oracle:
+    the four candidates equal the fp64 ones as a set (the SVD's orientation, hence their order, is free), the selected
+    pose equals the oracle's vote winner over the device's inlier mask, and points outside the mask are (0, 0, 0, 1)."""
+    torch = torch_cuda
+    K, Kinv = O.reference_K()
+    H = 2048
+    scenes = [O.synthetic_pair(n, seed=1000 * seed + b) for b in range(B)]
+    h = pkg.BatchedPairs(K, Kinv, B, n, H)
+    h.set_option(1, 0)
+    h.set_option(3, 1)
+    h.run_device(torch.from_numpy(np.stack([s["px"] for s in scenes])).cuda(), H, seed, THR)
+    E, Pg, ind = h.get_E(), h.get_poses(), h.get_pose_index()
+    for b in range(B):
+        xg = gpu_x(h, b)
+        mask = h.get_inlier_mask(b).cpu().numpy().astype(bool)
+        assert np.array_equal(mask, O.sampson_mask_f32(E[b], xg, THR))
+        Po = O.pose_candidates(E[b].astype(np.float64), compat=False)
+        assert O.match_candidate_set(Pg[b], Po, tol=1e-4) is not None, (b, np.abs(Pg[b] - Po).max())
+        votes = O.cheirality_votes(xg, Po, mask)
+        top = sorted(votes)
+        assert top[3] - top[2] > 0.01 * sum(votes), votes          # a clear winner, so the pose is pinned below
+        assert np.abs(Pg[b][ind[b]] - Po[int(np.argmax(votes))]).max() < 1e-4, (b, int(ind[b]), votes)
+        pts = h.get_points_host(b)
+        assert np.all(pts[:3, ~mask] == 0) and np.all(pts[3] == 1)
+        ref = O.triangulate(xg[mask], Pg[b][ind[b]].astype(np.float64))
+        rel = np.abs(pts[:3, mask] - ref[:3]).max(axis=0) / np.maximum(np.abs(ref[:3]).max(axis=0), 1e-3)
+        assert np.median(rel) <= 1e-6 and np.mean(rel < 1e-3) >= 0.99, (b, np.median(rel), np.mean(rel < 1e-3))
+    h.close()
+
+
 def test_batched_pairs_equal_single_pairs(pkg, O, torch_cuda):
     torch = torch_cuda
     K, Kinv = O.reference_K()
@@ -393,7 +427,13 @@ def test_full_size_properties_config2(pkg, O, oracle_c, torch_cuda):
     c64, amb = counts_f64(oracle_c, Enp, xg)
     diff = np.abs(got - c64)
     assert np.all(diff <= amb)
+    # ALL 65,536 candidates against the fp64 null vectors of the same rows
+    d = O.e_distance(Enp, O.hypotheses(xg, O.sample_indices(1237, H, n)))
+    assert np.mean(d < 1e-4) >= 0.995, f"{np.mean(d < 1e-4)} of hypotheses within 1e-4"
+    assert np.median(d) < 1e-6
     rec = {"config": "BASELINE config 2: 10,000 correspondences x 65,536 hypotheses, seed 1237, thr 1e-6", "band_rel": BAND,
+           "E_within_1e-4": float(np.mean(d < 1e-4)), "E_within_1e-6": float(np.mean(d < 1e-6)),
+           "E_median_distance": float(np.median(d)),
            "hypotheses": int(H), "evaluations": int(H) * n, "sum_borderline": int(amb.sum()), "sum_abs_diff_vs_fp64": int(diff.sum()),
            "max_abs_diff_vs_fp64": int(diff.max()), "hypotheses_with_any_diff": int((diff > 0).sum()),
            "fp32_port_bit_exact": True, "winner_fp32": [int(bi[0]), int(bc[0])],
