@@ -17,20 +17,45 @@ using namespace sfmb200;
 
 static thread_local char g_err[512] = "";
 
-static int fail(int code, const char* fmt, const char* detail = "") {
-    snprintf(g_err, sizeof(g_err), fmt, detail);
+static int fail(int code, const char* msg) {
+    snprintf(g_err, sizeof(g_err), "%s", msg);
     return code;
 }
-#define CK(call)                                                                     \
-    do {                                                                             \
-        cudaError_t e_ = (call);                                                     \
-        if (e_ != cudaSuccess) return fail(SFMB200_ERR_CUDA, #call ": %s", cudaGetErrorString(e_)); \
+static int fail_cuda(const char* what, cudaError_t e) {
+    snprintf(g_err, sizeof(g_err), "%s: %s", what, cudaGetErrorString(e));
+    return SFMB200_ERR_CUDA;
+}
+#define CK(call)                                           \
+    do {                                                   \
+        cudaError_t e_ = (call);                           \
+        if (e_ != cudaSuccess) return fail_cuda(#call, e_); \
     } while (0)
-#define CKL()                                                                        \
-    do {                                                                             \
-        cudaError_t e_ = cudaGetLastError();                                         \
-        if (e_ != cudaSuccess) return fail(SFMB200_ERR_CUDA, "kernel launch: %s", cudaGetErrorString(e_)); \
+#define CKL()                                                        \
+    do {                                                             \
+        cudaError_t e_ = cudaGetLastError();                         \
+        if (e_ != cudaSuccess) return fail_cuda("kernel launch", e_); \
     } while (0)
+
+// What s.E holds.
+enum class Held { nothing, essential, homography };
+
+// Which results of earlier calls the handle holds (include/sfmb200.h, "handle state").  Entry points check their
+// prerequisites with need() and change the record only through these transitions.
+struct HandleState {
+    bool points;        // correspondences are ingested
+    Held E;
+    bool candidates;    // the candidate arena holds hypotheses [h_begin, h_begin + H) of the last estimate, with counts
+    bool pose;          // pose candidates of the current E
+    bool chain;         // chain_views ran on the current reconstruction
+    void new_points() { points = true; chain = false; }     // the chained reconstruction belonged to the old ones
+    void lose_points() { points = false; }
+    void estimate(Held model) { E = model; candidates = true; pose = chain = false; }
+    void lose_candidates() { candidates = false; }
+    void new_E() { E = Held::essential; pose = chain = false; }
+    void lose_essential() { if (E == Held::essential) E = Held::nothing; }
+    void poses() { pose = true; }
+    void chained() { chain = true; }
+};
 
 struct sfmb200_handle {
     DeviceState s;
@@ -41,9 +66,9 @@ struct sfmb200_handle {
     GbaState gba;
     void* gba_arena;       // lazily allocated by sfmb200_bundle_adjust_global
     float* gba_stats;      // device [8] statistics of the last global adjustment
-    bool have_chain;       // chain_views ran on the current reconstruction
-    void* staging_in;      // lazily allocated: device copy of pageable host input
-    void* staging_out;     // lazily allocated: compact device copy of the points for host output
+    HandleState st;
+    float* px_staging;     // lazily allocated: device copy of pageable host input
+    float* pack_points;    // lazily allocated: device [B][4][n] compact copy of the triangulated points (run_host results)
     void* ba_arena;        // lazily allocated by sfmb200_bundle_adjust (6 floats + 1 byte per correspondence)
     MgPeers mg;            // multi-GPU peer exchange (mg.cu); mg.world == 0 until sfmb200_mg_init
     void* mg_local;        // this rank's exchange buffer (cudaMalloc, exported through CUDA IPC)
@@ -55,10 +80,6 @@ struct sfmb200_handle {
     long long mg_timeout_cycles;
     cudaStream_t stream;
     bool own_stream;
-    cudaStream_t aux_stream;       // side stream of the batched pipeline (hypothesis generation of later chunks runs under the
-    cudaEvent_t ev_fork;           // scoring of earlier ones); created on first use
-    cudaEvent_t ev_chunk[16];
-    int pipeline_chunks;           // SFMB200_OPT_BATCH_PIPELINE: -1 auto, 0 / 1 off, 2..16 chunks
     int device;
     int sms;               // SM count of the handle's device (cached at create)
     int compat;
@@ -67,17 +88,14 @@ struct sfmb200_handle {
     int hyp_solver;
     int small_path;        // SFMB200_OPT_SMALL_PATH: -1 auto, 0 never, 1 whenever eligible
     long long small_evals; // auto: use the fused single-launch path when n * H is at most this
-    int model;             // what s.E holds: 0 essential matrix, 1 homography (find_homography)
     // state of the last estimate
     int H;            // hypotheses in the local slice
     int h_begin;
     float thr;
-    bool have_points, have_E, have_candidates, have_pose;
     ScorePlan plan;
     int64_t launches;
     int* filter_scratch;   // [n_max / 256 + 2] per-CTA counts / offsets of the filtered ingest
     float* pack_header;    // device [B][32]: E 9, selected P 16, pose index, inliers, best index (run_host results)
-    float* pack_points;    // device [B][4][n] compact copy of the triangulated points
     float* host_header;    // pinned mirror of pack_header
     int* adapt;            // device [4]: adaptive termination flag, hypotheses used, pairs unsatisfied, spare
     void* arena;
@@ -120,31 +138,105 @@ struct DeviceScope {
         if (switched) cudaSetDevice(prev);
     }
 };
-#define ENTER(h)                                                                                          \
-    DeviceScope scope_(h);                                                                                \
-    if (scope_.err != cudaSuccess) return fail(SFMB200_ERR_CUDA, "cannot make the handle's device current: %s", cudaGetErrorString(scope_.err))
+#define ENTER(h)        \
+    DeviceScope scope_(h); \
+    if (scope_.err != cudaSuccess) return fail_cuda("cannot make the handle's device current", scope_.err)
+// ENTER for the entry points that refuse a null handle
+#define ENTER_HANDLE(h) \
+    ENTER(h);           \
+    if (!h) return fail(SFMB200_ERR_ARG, "null handle")
+
+// Prerequisites of an entry point: need() refuses the call with SFMB200_ERR_STATE and `msg` unless the handle holds all.
+constexpr unsigned NEED_POINTS = 1;
+constexpr unsigned NEED_ESSENTIAL = 2;      // s.E holds an essential matrix
+constexpr unsigned NEED_MODEL = 4;          // s.E holds an essential matrix or a homography
+constexpr unsigned NEED_POSE = 8;
+constexpr unsigned NEED_CHAIN = 16;
+constexpr unsigned NEED_CANDIDATES = 32;
+static int need(const sfmb200_handle* h, unsigned what, const char* msg) {
+    const HandleState& st = h->st;
+    const unsigned held = (st.points ? NEED_POINTS : 0u) | (st.E == Held::essential ? NEED_ESSENTIAL : 0u) |
+                          (st.E != Held::nothing ? NEED_MODEL : 0u) | (st.pose ? NEED_POSE : 0u) | (st.chain ? NEED_CHAIN : 0u) |
+                          (st.candidates ? NEED_CANDIDATES : 0u);
+    return (held & what) == what ? SFMB200_OK : fail(SFMB200_ERR_STATE, msg);
+}
+
+// Inlier threshold of the stages that follow an estimate: the last estimate's, or the reference's literal (sfm.cu:220)
+// while none has set one.
+static float stage_thr(const sfmb200_handle* h) { return h->thr > 0 ? h->thr : 1e-6f; }
+
+static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// An arena is written once, as a layout: a function that calls carve(&dst, count) for every buffer in it.  The layout
+// runs twice, first to size the allocation (every buffer 256-byte aligned), then to point each dst into it.
+struct Carver {
+    char* base;       // nullptr while sizing
+    size_t bytes;
+    template <typename T>
+    void operator()(T** dst, size_t count) {
+        if (base) *dst = (T*)(base + bytes);
+        bytes = align_up(bytes + count * sizeof(T), 256);
+    }
+};
+template <typename Layout>
+static cudaError_t alloc_arena(void** arena, size_t* bytes, Layout layout) {
+    Carver size = {nullptr, 0};
+    layout(size);
+    cudaError_t e = cudaMalloc(arena, size.bytes);
+    if (e != cudaSuccess) return e;
+    Carver place = {(char*)*arena, 0};
+    layout(place);
+    *bytes = size.bytes;
+    return cudaSuccess;
+}
+// Scratch that only some workflows need: allocated and zeroed (on the handle's stream) by the first call that uses it.
+template <typename Layout>
+static int lazy_arena(sfmb200_handle* h, void** arena, Layout layout) {
+    if (*arena) return SFMB200_OK;
+    size_t bytes = 0;
+    CK(alloc_arena(arena, &bytes, layout));
+    CK(cudaMemsetAsync(*arena, 0, bytes, h->stream));
+    return SFMB200_OK;
+}
+
+// Frees whatever the handle holds: sfmb200_destroy, and sfmb200_create when it fails part-way.
+static void release(sfmb200_handle* h) {
+    if (h->own_stream) cudaStreamDestroy(h->stream);
+    if (h->host_header) cudaFreeHost(h->host_header);
+    if (h->prof_ev) {
+        for (int i = 0; i < PROF_RING; i++)
+            for (int k = 0; k < 8; k++) cudaEventDestroy(h->prof_ev[i][k]);
+        delete[] h->prof_ev;
+        delete[] h->prof_mask;
+    }
+    for (void* p : {h->arena, h->chain_arena, h->gba_arena, h->ba_arena, (void*)h->px_staging, (void*)h->pack_points})
+        if (p) cudaFree(p);
+    delete h;
+}
 
 extern "C" {
 
 const char* sfmb200_last_error(void) { return g_err; }
 int sfmb200_version(void) { return 100; }
 
-static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
 int sfmb200_create(const float K[9], const float Kinv[9], int pairs, int max_points, int max_hyp, sfmb200_t** out) {
-    if (!K || !Kinv || !out) return fail(SFMB200_ERR_ARG, "null argument%s");
-    if (pairs < 1 || max_points < 8 || max_hyp < 1) return fail(SFMB200_ERR_ARG, "pairs >= 1, max_points >= 8, max_hypotheses >= 1 required%s");
-    if (pairs > 65535) return fail(SFMB200_ERR_ARG, "at most 65535 pairs per handle (grid.y / grid.z limit)%s");
+    if (!K || !Kinv || !out) return fail(SFMB200_ERR_ARG, "null argument");
+    if (pairs < 1 || max_points < 8 || max_hyp < 1) return fail(SFMB200_ERR_ARG, "pairs >= 1, max_points >= 8, max_hypotheses >= 1 required");
+    if (pairs > 65535) return fail(SFMB200_ERR_ARG, "at most 65535 pairs per handle (grid.y / grid.z limit)");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();
-        return fail(SFMB200_ERR_NODEVICE, "no CUDA device: sfmb200 has no CPU fallback%s");
+        return fail(SFMB200_ERR_NODEVICE, "no CUDA device: sfmb200 has no CPU fallback");
     }
     sfmb200_handle* h = new (std::nothrow) sfmb200_handle();
-    if (!h) return fail(SFMB200_ERR_ARG, "out of host memory%s");
+    if (!h) return fail(SFMB200_ERR_ARG, "out of host memory");
     memset(h, 0, sizeof(*h));
-    CK(cudaGetDevice(&h->device));
-    CK(cudaDeviceGetAttribute(&h->sms, cudaDevAttrMultiProcessorCount, h->device));
+    cudaError_t e = cudaGetDevice(&h->device);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&h->sms, cudaDevAttrMultiProcessorCount, h->device);
+    if (e != cudaSuccess) {
+        release(h);
+        return fail_cuda("create: device query", e);
+    }
     DeviceState& s = h->s;
     s.B = pairs;
     s.n_max = max_points;
@@ -155,81 +247,55 @@ int sfmb200_create(const float K[9], const float Kinv[9], int pairs, int max_poi
     s.tiles_max = s.h_stride / SCORE_MIN_TILE;
     memcpy(s.K, K, sizeof(float) * 9);
     memcpy(s.Kinv, Kinv, sizeof(float) * 9);
-    // one arena, carved with 256-byte alignment
-    size_t B = pairs, off = 0;
-    auto carve = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-    size_t o_corr = carve(B * s.n_stride * sizeof(float4));
-    size_t o_cs = carve(B * s.n_stride * sizeof(float4));
-    size_t o_ec = carve(B * 9 * (size_t)s.h_stride * sizeof(float));
-    size_t o_cnt = carve(B * (size_t)s.h_stride * sizeof(int));
-    size_t o_td = carve(B * (size_t)s.tiles_max * sizeof(int));
-    size_t o_best = carve(B * sizeof(unsigned long long));
-    size_t o_E = carve(B * 9 * sizeof(float));
-    size_t o_bi = carve(B * sizeof(int));
-    size_t o_bc = carve(B * sizeof(int));
-    size_t o_P = carve(B * 64 * sizeof(float));
-    size_t o_pi = carve(B * sizeof(int));
-    size_t o_pts = carve(B * 4 * (size_t)s.n_stride * sizeof(float));
-    size_t o_tc = carve(B * sizeof(int));
-    size_t o_vote = carve(B * 8 * sizeof(int));
-    size_t o_fs = carve(((size_t)max_points / 256 + 2) * sizeof(int));
-    size_t o_ph = carve(B * 32 * sizeof(float));
-    size_t o_ad = carve(4 * sizeof(int));
-    const int refit_blocks = 64;
-    size_t o_rc = carve(B * 9 * sizeof(float));
-    size_t o_rT = carve(B * 8 * sizeof(float));
-    size_t o_rf = carve(B * 4 * sizeof(int));
-    size_t o_ri = carve(B * sizeof(int));
-    size_t o_rm = carve(B * refit_blocks * 8 * sizeof(float));
-    size_t o_rg = carve(B * refit_blocks * 45 * sizeof(float));
-    cudaError_t e = cudaMalloc(&h->arena, off);
-    if (e != cudaSuccess) {
-        delete h;
-        return fail(SFMB200_ERR_CUDA, "cudaMalloc(arena): %s", cudaGetErrorString(e));
-    }
-    char* base = (char*)h->arena;
-    s.corr = (float4*)(base + o_corr);
-    s.corr_s = (float4*)(base + o_cs);
     s.pt_scale = make_thr_scale(1e-6f).ik;     // the reference's threshold literal (sfm.cu:220) until told otherwise
-    s.px = nullptr;            // staging for pageable host input: allocated on first use (ensure_staging)
-    s.Ecand = (float*)(base + o_ec);
-    s.counts = (int*)(base + o_cnt);
-    s.tile_done = (int*)(base + o_td);
-    s.best = (unsigned long long*)(base + o_best);
-    s.E = (float*)(base + o_E);
-    s.best_idx = (int*)(base + o_bi);
-    s.best_count = (int*)(base + o_bc);
-    s.P = (float*)(base + o_P);
-    s.P_ind = (int*)(base + o_pi);
-    s.points = (float*)(base + o_pts);
-    s.tri_count = (int*)(base + o_tc);
-    s.vote = (int*)(base + o_vote);
-    h->filter_scratch = (int*)(base + o_fs);
-    h->pack_header = (float*)(base + o_ph);
-    h->pack_points = nullptr;  // staging for host output: allocated on first use (ensure_staging)
-    h->adapt = (int*)(base + o_ad);
-    h->ba.persistent = 1;      // the bundle-adjustment scratch itself is allocated on first use (ensure_ba_arena)
-    h->refit.cand = (float*)(base + o_rc);
-    h->refit.T = (float*)(base + o_rT);
-    h->refit.flags = (int*)(base + o_rf);
-    h->refit.iters_done = (int*)(base + o_ri);
-    h->refit.mom_part = (float*)(base + o_rm);
-    h->refit.gram_part = (float*)(base + o_rg);
-    h->refit.max_blocks = refit_blocks;
-    e = cudaMemset(h->arena, 0, off);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaMallocHost((void**)&h->host_header, B * 32 * sizeof(float));
+    const size_t B = pairs;
+    RefitState& r = h->refit;
+    r.max_blocks = 64;
+    size_t bytes = 0;
+    e = alloc_arena(&h->arena, &bytes, [&](Carver& carve) {
+        carve(&s.corr, B * s.n_stride);
+        carve(&s.corr_s, B * s.n_stride);
+        carve(&s.Ecand, B * 9 * (size_t)s.h_stride);
+        carve(&s.counts, B * (size_t)s.h_stride);
+        carve(&s.tile_done, B * (size_t)s.tiles_max);
+        carve(&s.best, B);
+        carve(&s.E, B * 9);
+        carve(&s.best_idx, B);
+        carve(&s.best_count, B);
+        carve(&s.P, B * 64);
+        carve(&s.P_ind, B);
+        carve(&s.points, B * 4 * (size_t)s.n_stride);
+        carve(&s.tri_count, B);
+        carve(&s.vote, B * 8);
+        carve(&h->filter_scratch, (size_t)max_points / 256 + 2);
+        carve(&h->pack_header, B * 32);
+        carve(&h->adapt, 4);
+        carve(&r.cand, B * 9);
+        carve(&r.T, B * 8);
+        carve(&r.flags, B * 4);
+        carve(&r.iters_done, B);
+        carve(&r.mom_part, B * r.max_blocks * 8);
+        carve(&r.gram_part, B * r.max_blocks * 45);
+    });
     if (e != cudaSuccess) {
-        cudaFree(h->arena);
-        delete h;
-        return fail(SFMB200_ERR_CUDA, "create: %s", cudaGetErrorString(e));
+        release(h);
+        return fail_cuda("cudaMalloc(arena)", e);
     }
-    h->own_stream = true;
+    h->ba.persistent = 1;      // the bundle-adjustment scratch itself is allocated on first use (ensure_ba_arena)
+    e = cudaMemset(h->arena, 0, bytes);
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
+    if (e == cudaSuccess) {
+        h->own_stream = true;
+        e = cudaMallocHost((void**)&h->host_header, B * 32 * sizeof(float));
+    }
+    if (e != cudaSuccess) {
+        release(h);
+        return fail_cuda("create", e);
+    }
     h->compat = 1;
     h->hyp_solver = 1;     // Cholesky projector: same parity as the Jacobi eigensolve, 3.5-4.4x faster (profiles/)
     h->score_variant = -1;
     h->tri_inliers_only = 0;
-    h->pipeline_chunks = -1;
     h->small_path = -1;
     h->small_evals = 2500000;      // crossover with the five-launch path on B200: device time ~1.5e6, call latency ~2.5e6 (profiles/r02_small_path.md)
     *out = h;
@@ -241,62 +307,38 @@ int sfmb200_destroy(sfmb200_t* h) {
     if (!h) return SFMB200_OK;
     cudaStreamSynchronize(h->stream);
     sfmb200_mg_close(h);          // unmaps the peers' exchange buffers; needs the stream, so before it goes
-    if (h->aux_stream) {
-        cudaStreamDestroy(h->aux_stream);
-        cudaEventDestroy(h->ev_fork);
-        for (int i = 0; i < 16; i++) cudaEventDestroy(h->ev_chunk[i]);
-    }
-    if (h->own_stream) cudaStreamDestroy(h->stream);
-    if (h->host_header) cudaFreeHost(h->host_header);
-    if (h->prof_ev) {
-        for (int i = 0; i < PROF_RING; i++)
-            for (int k = 0; k < 8; k++) cudaEventDestroy(h->prof_ev[i][k]);
-        delete[] h->prof_ev;
-        delete[] h->prof_mask;
-    }
-    cudaFree(h->arena);
-    if (h->chain_arena) cudaFree(h->chain_arena);
-    if (h->gba_arena) cudaFree(h->gba_arena);
-    if (h->ba_arena) cudaFree(h->ba_arena);
-    if (h->staging_in) cudaFree(h->staging_in);
-    if (h->staging_out) cudaFree(h->staging_out);
-    delete h;
+    release(h);
     return SFMB200_OK;
 }
 
 int sfmb200_set_option(sfmb200_t* h, int option, int value) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
+    ENTER_HANDLE(h);
     switch (option) {
         case SFMB200_OPT_COMPAT: h->compat = value ? 1 : 0; break;
         case SFMB200_OPT_SCORE_VARIANT:
-            if (value < -1 || value >= score_num_variants()) return fail(SFMB200_ERR_ARG, "score variant out of range%s");
+            if (value < -1 || value >= score_num_variants()) return fail(SFMB200_ERR_ARG, "score variant out of range");
             h->score_variant = value;
             break;
         case SFMB200_OPT_TRI_INLIERS_ONLY: h->tri_inliers_only = value ? 1 : 0; break;
         case SFMB200_OPT_HYP_SOLVER:
-            if (value < 0 || value > 1) return fail(SFMB200_ERR_ARG, "hypothesis solver must be 0 (Jacobi) or 1 (Cholesky projector)%s");
+            if (value < 0 || value > 1) return fail(SFMB200_ERR_ARG, "hypothesis solver must be 0 (Jacobi) or 1 (Cholesky projector)");
             h->hyp_solver = value;
             break;
         case SFMB200_OPT_BA_PERSISTENT: h->ba.persistent = value ? 1 : 0; break;
-        case SFMB200_OPT_BATCH_PIPELINE:
-            if (value < -1 || value > 16) return fail(SFMB200_ERR_ARG, "batch pipeline chunks must be -1 (auto), 0 / 1 (off) or 2..16%s");
-            h->pipeline_chunks = value;
-            break;
         case SFMB200_OPT_SAMPLER:
-            if (value < 0 || value > 1) return fail(SFMB200_ERR_ARG, "sampler must be 0 (independent subsets) or 1 (disjoint permutation)%s");
+            if (value < 0 || value > 1) return fail(SFMB200_ERR_ARG, "sampler must be 0 (independent subsets) or 1 (disjoint permutation)");
             h->s.sampler = value;
             break;
         case SFMB200_OPT_SCORE_METRIC:
-            if (value < 0 || value > 1) return fail(SFMB200_ERR_ARG, "score metric must be 0 (Sampson error) or 1 (symmetric epipolar distance)%s");
+            if (value < 0 || value > 1) return fail(SFMB200_ERR_ARG, "score metric must be 0 (Sampson error) or 1 (symmetric epipolar distance)");
             h->s.metric = value;
             break;
         case SFMB200_OPT_SMALL_PATH:
-            if (value < -1 || value > 1) return fail(SFMB200_ERR_ARG, "small path must be -1 (auto), 0 (never) or 1 (whenever eligible)%s");
+            if (value < -1 || value > 1) return fail(SFMB200_ERR_ARG, "small path must be -1 (auto), 0 (never) or 1 (whenever eligible)");
             h->small_path = value;
             break;
         case SFMB200_OPT_SMALL_PATH_EVALS:
-            if (value < 0) return fail(SFMB200_ERR_ARG, "evaluation limit must be >= 0%s");
+            if (value < 0) return fail(SFMB200_ERR_ARG, "evaluation limit must be >= 0");
             h->small_evals = value;
             break;
         case SFMB200_OPT_PROFILE:
@@ -311,14 +353,13 @@ int sfmb200_set_option(sfmb200_t* h, int option, int value) {
             h->prof_cur = 0;
             if (h->prof_mask) memset(h->prof_mask, 0, PROF_RING);
             break;
-        default: return fail(SFMB200_ERR_ARG, "unknown option%s");
+        default: return fail(SFMB200_ERR_ARG, "unknown option");
     }
     return SFMB200_OK;
 }
 
 int sfmb200_set_stream(sfmb200_t* h, void* stream) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
+    ENTER_HANDLE(h);
     if (h->own_stream) {
         cudaStreamSynchronize(h->stream);
         cudaStreamDestroy(h->stream);
@@ -329,15 +370,14 @@ int sfmb200_set_stream(sfmb200_t* h, void* stream) {
 }
 
 int sfmb200_synchronize(sfmb200_t* h) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
+    ENTER_HANDLE(h);
     CK(cudaStreamSynchronize(h->stream));
     return SFMB200_OK;
 }
 
 static int check_n(sfmb200_t* h, const void* p, int n) {
-    if (!h || !p) return fail(SFMB200_ERR_ARG, "null argument%s");
-    if (n < 8 || n > h->s.n_max) return fail(SFMB200_ERR_ARG, "n must be in [8, max_points]%s");
+    if (!h || !p) return fail(SFMB200_ERR_ARG, "null argument");
+    if (n < 8 || n > h->s.n_max) return fail(SFMB200_ERR_ARG, "n must be in [8, max_points]");
     return SFMB200_OK;
 }
 
@@ -345,13 +385,12 @@ int sfmb200_set_points_sift(sfmb200_t* h, const void* d_sift, int n) {
     ENTER(h);
     int rc = check_n(h, d_sift, n);
     if (rc) return rc;
-    if (h->s.B != 1) return fail(SFMB200_ERR_ARG, "SiftPoint ingest needs pairs == 1%s");
+    if (h->s.B != 1) return fail(SFMB200_ERR_ARG, "SiftPoint ingest needs pairs == 1");
     h->s.n = n;
     launch_ingest_sift(h->s, d_sift, n, h->stream);
     CKL();
     h->launches++;
-    h->have_points = true;
-    h->have_chain = false;       // the chained reconstruction belonged to the previous correspondences
+    h->st.new_points();
     return SFMB200_OK;
 }
 int sfmb200_set_points_sift_filtered(sfmb200_t* h, const void* d_sift, int n, float min_score, float max_ambiguity,
@@ -359,8 +398,8 @@ int sfmb200_set_points_sift_filtered(sfmb200_t* h, const void* d_sift, int n, fl
     ENTER(h);
     int rc = check_n(h, d_sift, n);
     if (rc) return rc;
-    if (h->s.B != 1) return fail(SFMB200_ERR_ARG, "SiftPoint ingest needs pairs == 1%s");
-    h->have_points = false;
+    if (h->s.B != 1) return fail(SFMB200_ERR_ARG, "SiftPoint ingest needs pairs == 1");
+    h->st.lose_points();
     launch_ingest_sift_filtered(h->s, d_sift, n, min_score, max_ambiguity, h->filter_scratch, d_kept_index, h->stream);
     CKL();
     h->launches += 3;
@@ -370,10 +409,9 @@ int sfmb200_set_points_sift_filtered(sfmb200_t* h, const void* d_sift, int n, fl
     CK(cudaMemcpyAsync(&kept, h->filter_scratch + blocks, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (h_kept) *h_kept = kept;
-    if (kept < 8) return fail(SFMB200_ERR_STATE, "fewer than 8 correspondences survive the match filter%s");
+    if (kept < 8) return fail(SFMB200_ERR_STATE, "fewer than 8 correspondences survive the match filter");
     h->s.n = kept;
-    h->have_points = true;
-    h->have_chain = false;       // the chained reconstruction belonged to the previous correspondences
+    h->st.new_points();
     return SFMB200_OK;
 }
 // `scale` > 0: the ingest also commits a new threshold scale for the scaled copies (run_device / run_host pass the
@@ -389,38 +427,25 @@ static int ingest_xy(sfmb200_t* h, const float* d_px, int n, float scale) {
     prof_mark(h, 1);
     CKL();
     h->launches++;
-    h->have_points = true;
-    h->have_chain = false;       // the chained reconstruction belonged to the previous correspondences
+    h->st.new_points();
     return SFMB200_OK;
 }
 int sfmb200_set_points_xy(sfmb200_t* h, const float* d_px, int n) {
     ENTER(h);
     return ingest_xy(h, d_px, n, 0.0f);
 }
-// Device staging for host buffers that the kernels cannot reach directly (pageable, or larger than the zero-copy
-// limit): allocated on first use, so device-resident workflows (run_device, the batched configs) never pay for it.
-static int ensure_staging(sfmb200_handle* h, bool in, bool out) {
-    if (in && !h->staging_in) {
-        CK(cudaMalloc(&h->staging_in, (size_t)h->s.B * h->s.n_stride * 4 * sizeof(float)));
-        h->s.px = (float*)h->staging_in;
-    }
-    if (out && !h->staging_out) {
-        CK(cudaMalloc(&h->staging_out, (size_t)h->s.B * 4 * (size_t)h->s.n_max * sizeof(float)));
-        h->pack_points = (float*)h->staging_out;
-    }
+// Device copy of host input that the kernels cannot reach directly (pageable, or larger than the zero-copy limit): the
+// staging buffer is allocated on first use, so device-resident workflows (run_device, the batched configs) never pay for it.
+static int stage_input(sfmb200_handle* h, const float* h_px, int n) {
+    if (!h->px_staging) CK(cudaMalloc(&h->px_staging, (size_t)h->s.B * h->s.n_stride * 4 * sizeof(float)));
+    CK(cudaMemcpyAsync(h->px_staging, h_px, (size_t)h->s.B * n * 4 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     return SFMB200_OK;
-}
-
-static int ingest_xy_host(sfmb200_t* h, const float* h_px, int n, float scale) {
-    int rc = check_n(h, h_px, n);
-    if (rc) return rc;
-    if ((rc = ensure_staging(h, true, false))) return rc;
-    CK(cudaMemcpyAsync(h->s.px, h_px, (size_t)h->s.B * n * 4 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    return ingest_xy(h, h->s.px, n, scale);
 }
 int sfmb200_set_points_xy_host(sfmb200_t* h, const float* h_px, int n) {
     ENTER(h);
-    return ingest_xy_host(h, h_px, n, 0.0f);
+    if (int rc = check_n(h, h_px, n)) return rc;
+    if (int rc = stage_input(h, h_px, n)) return rc;
+    return ingest_xy(h, h->px_staging, n, 0.0f);
 }
 int sfmb200_set_points_normalised(sfmb200_t* h, const float* d_x, int n) {
     ENTER(h);
@@ -430,8 +455,7 @@ int sfmb200_set_points_normalised(sfmb200_t* h, const float* d_x, int n) {
     launch_ingest_normalised(h->s, d_x, n, h->stream);
     CKL();
     h->launches++;
-    h->have_points = true;
-    h->have_chain = false;       // the chained reconstruction belonged to the previous correspondences
+    h->st.new_points();
     return SFMB200_OK;
 }
 
@@ -461,7 +485,7 @@ static ScorePlan plan_essential(const sfmb200_handle* h, int n, int H) {
 // hypotheses fit one cluster's shared memory; `pose`: the call also runs the pose stage, which the fused kernel
 // implements in reference (compat) semantics only.  Not used while per-stage events are being recorded.
 constexpr int SMALL_PATH_MAX_PAIRS = 4;
-static bool small_path_ok(const sfmb200_handle* h, int H, bool pose) {
+static bool small_path_ok(const sfmb200_handle* h, int n, int H, bool pose) {
     if (h->small_path == 0 || h->profile || h->hyp_solver != 1 || h->s.skip != nullptr || h->s.metric != 0) return false;
     if (h->score_variant >= 0 && h->small_path != 1) return false;      // the caller asked for a specific scoring kernel
     if (pose && !h->compat) return false;
@@ -470,24 +494,23 @@ static bool small_path_ok(const sfmb200_handle* h, int H, bool pose) {
     // automatic: one 16-CTA cluster per pair fills a GPC, so beyond a handful of pairs the clusters queue up behind each other
     // while the general path's kernels spread every pair over the whole GPU (measured: 4 pairs 28.7 vs 30.7 us, 8 pairs 50 vs 35 us)
     if (h->s.B > SMALL_PATH_MAX_PAIRS) return false;
-    return (long long)h->s.n * (long long)H <= h->small_evals;
+    return (long long)n * (long long)H <= h->small_evals;
 }
 
 int sfmb200_estimate_e_slice(sfmb200_t* h, const int32_t* d_idx, int H_total, int h_begin, int H, uint64_t seed,
                              float thr) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!h->have_points) return fail(SFMB200_ERR_STATE, "estimate_e before set_points%s");
+    ENTER_HANDLE(h);
+    if (int rc = need(h, NEED_POINTS, "estimate_e before set_points")) return rc;
     if (H < 1 || H > h->s.h_max || h_begin < 0 || (long long)h_begin + H > (long long)H_total)
-        return fail(SFMB200_ERR_ARG, "hypothesis slice out of range / above max_hypotheses%s");
-    if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive%s");
+        return fail(SFMB200_ERR_ARG, "hypothesis slice out of range / above max_hypotheses");
+    if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive");
     if (!d_idx && h->s.sampler == 1 && 8ll * H_total > (long long)h->s.n)
-        return fail(SFMB200_ERR_ARG, "the disjoint-permutation sampler needs 8 * H_total <= n (the reference uses H = N / 8)%s");
+        return fail(SFMB200_ERR_ARG, "the disjoint-permutation sampler needs 8 * H_total <= n (the reference uses H = N / 8)");
     h->H = H;
     h->h_begin = h_begin;
     h->thr = thr;
     if (int rc = ensure_scaled(h, make_thr_scale(thr).ik)) return rc;
-    if (small_path_ok(h, H, false)) {
+    if (small_path_ok(h, h->s.n, H, false)) {
         // hypothesis generation + scoring + arg-max + selection in one cluster launch
         CK(launch_small_path(h->s, nullptr, d_idx, (long long)H_total * 8, H, h_begin, seed, thr, h->compat, 0, SMALL_ESTIMATE, h->stream));
         memset(&h->plan, 0, sizeof(h->plan));
@@ -506,20 +529,15 @@ int sfmb200_estimate_e_slice(sfmb200_t* h, const int32_t* d_idx, int H_total, in
         CKL();
         h->launches += 3;
     }
-    h->have_candidates = true;
-    h->have_E = true;
-    h->have_pose = false;
-    h->have_chain = false;
-    h->model = 0;
+    h->st.estimate(Held::essential);
     return SFMB200_OK;
 }
 
 int sfmb200_find_homography(sfmb200_t* h, int loops, uint64_t seed, float thresh, float* h_H, int32_t* h_matches) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!h->have_points) return fail(SFMB200_ERR_STATE, "find_homography before set_points%s");
-    if (loops < 1 || loops > h->s.h_max) return fail(SFMB200_ERR_ARG, "loops out of range / above max_hypotheses%s");
-    if (!(thresh > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive%s");
+    ENTER_HANDLE(h);
+    if (int rc = need(h, NEED_POINTS, "find_homography before set_points")) return rc;
+    if (loops < 1 || loops > h->s.h_max) return fail(SFMB200_ERR_ARG, "loops out of range / above max_hypotheses");
+    if (!(thresh > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive");
     // `thresh` is in PIXELS like CudaSift's (matching.cu:953-996 runs on pixel coordinates), but the handle holds
     // K^-1-normalised coordinates.  For a camera with square pixels and no skew a pixel distance is exactly f times
     // a normalised one, so the test runs in normalised units with thresh / f and the result is mapped back with
@@ -529,7 +547,7 @@ int sfmb200_find_homography(sfmb200_t* h, int loops, uint64_t seed, float thresh
     const bool isotropic = f > 0.0f && fabsf(Kc[4] - f) <= 1e-6f * f && Kc[1] == 0.0f && Kc[3] == 0.0f && Kc[6] == 0.0f &&
                            Kc[7] == 0.0f && Kc[8] == 1.0f;
     if (!isotropic)
-        return fail(SFMB200_ERR_ARG, "find_homography needs K = [f 0 cx; 0 f cy; 0 0 1] (square pixels, no skew): the pixel threshold is applied as thresh / f%s");
+        return fail(SFMB200_ERR_ARG, "find_homography needs K = [f 0 cx; 0 f cy; 0 0 1] (square pixels, no skew): the pixel threshold is applied as thresh / f");
     const float thresh_n = thresh / f;
     const float thr2 = thresh_n * thresh_n;
     if (int rc = ensure_scaled(h, 1.0f)) return rc;      // the transfer-error test works on the unscaled coordinates
@@ -544,11 +562,7 @@ int sfmb200_find_homography(sfmb200_t* h, int loops, uint64_t seed, float thresh
     launch_select(h->s, 0, h->stream);
     CKL();
     h->launches += 3;
-    h->have_candidates = true;
-    h->have_E = false;        // s.E holds a homography now: the pose stages must not consume it
-    h->have_pose = false;
-    h->have_chain = false;
-    h->model = 1;
+    h->st.estimate(Held::homography);      // the pose stages must not consume it
     if (h_H) CK(cudaMemcpyAsync(h_H, h->s.E, (size_t)h->s.B * 9 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     if (h_matches) CK(cudaMemcpyAsync(h_matches, h->s.best_count, (size_t)h->s.B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     if (h_H || h_matches) CK(cudaStreamSynchronize(h->stream));
@@ -588,18 +602,17 @@ int sfmb200_estimate_e(sfmb200_t* h, const int32_t* d_idx, int H, uint64_t seed,
 // (counter-based sampler) or when d_idx rows are the same prefix.
 int sfmb200_estimate_e_adaptive(sfmb200_t* h, const int32_t* d_idx, int H_max, int first_round, int growth,
                                 uint64_t seed, float thr, float confidence, int32_t* h_used) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!h->have_points) return fail(SFMB200_ERR_STATE, "estimate_e before set_points%s");
-    if (H_max < 1 || first_round < 1 || growth < 2) return fail(SFMB200_ERR_ARG, "H_max >= 1, first_round >= 1, growth >= 2 required%s");
-    if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive%s");
-    if (!(confidence > 0.0f && confidence < 1.0f)) return fail(SFMB200_ERR_ARG, "confidence must be in (0, 1)%s");
+    ENTER_HANDLE(h);
+    if (int rc = need(h, NEED_POINTS, "estimate_e before set_points")) return rc;
+    if (H_max < 1 || first_round < 1 || growth < 2) return fail(SFMB200_ERR_ARG, "H_max >= 1, first_round >= 1, growth >= 2 required");
+    if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive");
+    if (!(confidence > 0.0f && confidence < 1.0f)) return fail(SFMB200_ERR_ARG, "confidence must be in (0, 1)");
     // every round must fit the candidate arena
     {
         long long lo = 0, hi = first_round;
         while (lo < H_max) {
             if (hi > H_max) hi = H_max;
-            if (hi - lo > h->s.h_max) return fail(SFMB200_ERR_ARG, "a round exceeds max_hypotheses of the handle%s");
+            if (hi - lo > h->s.h_max) return fail(SFMB200_ERR_ARG, "a round exceeds max_hypotheses of the handle");
             lo = hi;
             hi *= growth;
         }
@@ -630,11 +643,8 @@ int sfmb200_estimate_e_adaptive(sfmb200_t* h, const int32_t* d_idx, int H_max, i
     }
     // the decide kernel of each round publishes the running winner (E, index, count) from that round's arena
     h->thr = thr;
-    h->have_candidates = false;   // the candidate arena holds whichever round ran last, not [0, used)
-    h->have_E = true;
-    h->have_pose = false;
-    h->have_chain = false;
-    h->model = 0;
+    h->st.estimate(Held::essential);
+    h->st.lose_candidates();      // the candidate arena holds whichever round ran last, not [0, used)
     if (h_used) {
         CK(cudaMemcpyAsync(h_used, h->adapt + 1, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
@@ -653,9 +663,9 @@ int sfmb200_mg_handle_bytes(void) { return (int)sizeof(MgBlob); }
 
 int sfmb200_mg_init(sfmb200_t* h, int rank, int world, void* h_handle_out) {
     ENTER(h);
-    if (!h || !h_handle_out) return fail(SFMB200_ERR_ARG, "null argument%s");
-    if (world < 1 || world > MG_MAX_WORLD || rank < 0 || rank >= world) return fail(SFMB200_ERR_ARG, "bad rank / world (at most 16 ranks)%s");
-    if (h->mg_local) return fail(SFMB200_ERR_STATE, "mg_init called twice%s");
+    if (!h || !h_handle_out) return fail(SFMB200_ERR_ARG, "null argument");
+    if (world < 1 || world > MG_MAX_WORLD || rank < 0 || rank >= world) return fail(SFMB200_ERR_ARG, "bad rank / world (at most 16 ranks)");
+    if (h->mg_local) return fail(SFMB200_ERR_STATE, "mg_init called twice");
     const size_t bytes = mg_buffer_bytes(h->s.B, world);
     CK(cudaMalloc(&h->mg_local, bytes));
     CK(cudaMemset(h->mg_local, 0, bytes));
@@ -684,17 +694,17 @@ int sfmb200_mg_init(sfmb200_t* h, int rank, int world, void* h_handle_out) {
 
 int sfmb200_mg_set_timeout_ms(sfmb200_t* h, int ms) {
     ENTER(h);
-    if (!h || ms < 1) return fail(SFMB200_ERR_ARG, "timeout must be >= 1 ms%s");
-    if (!h->mg_local) return fail(SFMB200_ERR_STATE, "mg_set_timeout_ms before mg_init%s");
+    if (!h || ms < 1) return fail(SFMB200_ERR_ARG, "timeout must be >= 1 ms");
+    if (!h->mg_local) return fail(SFMB200_ERR_STATE, "mg_set_timeout_ms before mg_init");
     h->mg_timeout_cycles = (long long)ms * h->mg_clock_khz;
     return SFMB200_OK;
 }
 
 int sfmb200_mg_connect(sfmb200_t* h, const void* h_handles) {
     ENTER(h);
-    if (!h || !h_handles) return fail(SFMB200_ERR_ARG, "null argument%s");
-    if (!h->mg_local) return fail(SFMB200_ERR_STATE, "mg_connect before mg_init%s");
-    if (h->mg_connected) return fail(SFMB200_ERR_STATE, "mg_connect called twice%s");
+    if (!h || !h_handles) return fail(SFMB200_ERR_ARG, "null argument");
+    if (!h->mg_local) return fail(SFMB200_ERR_STATE, "mg_connect before mg_init");
+    if (h->mg_connected) return fail(SFMB200_ERR_STATE, "mg_connect called twice");
     const MgBlob* all = (const MgBlob*)h_handles;
     int ndev = 0;
     CK(cudaGetDeviceCount(&ndev));
@@ -708,11 +718,11 @@ int sfmb200_mg_connect(sfmb200_t* h, const void* h_handles) {
             CK(cudaGetDeviceProperties(&prop, d));
             if (memcmp(prop.uuid.bytes, all[r].uuid, 16) == 0) peer_dev = d;
         }
-        if (peer_dev < 0) return fail(SFMB200_ERR_ARG, "mg_connect: a peer's device is not visible to this process%s");
+        if (peer_dev < 0) return fail(SFMB200_ERR_ARG, "mg_connect: a peer's device is not visible to this process");
         if (peer_dev != h->device) {
             int native = 0;
             CK(cudaDeviceGetP2PAttribute(&native, cudaDevP2PAttrNativeAtomicSupported, h->device, peer_dev));
-            if (!native) return fail(SFMB200_ERR_STATE, "mg_connect: no native P2P atomics between this device and a peer (not NVLink-connected)%s");
+            if (!native) return fail(SFMB200_ERR_STATE, "mg_connect: no native P2P atomics between this device and a peer (not NVLink-connected)");
         }
         void* p = nullptr;
         CK(cudaIpcOpenMemHandle(&p, all[r].ipc, cudaIpcMemLazyEnablePeerAccess));
@@ -743,16 +753,15 @@ int sfmb200_mg_close(sfmb200_t* h) {
 // Every rank calls this with the same arguments on the same correspondences: scores its own slice of the
 // H_total hypotheses, exchanges the packed winners through peer memory and takes the global winner's E.
 int sfmb200_estimate_e_mg(sfmb200_t* h, const int32_t* d_idx, int H_total, uint64_t seed, float thr) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!h->mg_connected) return fail(SFMB200_ERR_STATE, "estimate_e_mg before mg_init / mg_connect%s");
+    ENTER_HANDLE(h);
+    if (!h->mg_connected) return fail(SFMB200_ERR_STATE, "estimate_e_mg before mg_init / mg_connect");
     if (*(volatile int*)h->mg_failed_host != 0) {
-        h->have_E = false;
-        h->have_candidates = false;
-        return fail(SFMB200_ERR_STATE, "the peer exchange timed out earlier (a rank is lost or late): sfmb200_mg_close + mg_init + mg_connect on every rank%s");
+        h->st.lose_essential();
+        h->st.lose_candidates();
+        return fail(SFMB200_ERR_STATE, "the peer exchange timed out earlier (a rank is lost or late): sfmb200_mg_close + mg_init + mg_connect on every rank");
     }
     const int world = h->mg.world, rank = h->mg.rank;
-    if (H_total < world) return fail(SFMB200_ERR_ARG, "fewer hypotheses than ranks%s");
+    if (H_total < world) return fail(SFMB200_ERR_ARG, "fewer hypotheses than ranks");
     const long long base = H_total / world, rem = H_total % world;
     const long long lo = rank * base + (rank < rem ? rank : rem), cnt = base + (rank < rem ? 1 : 0);
     int rc = sfmb200_estimate_e_slice(h, d_idx, H_total, (int)lo, (int)cnt, seed, thr);
@@ -761,7 +770,7 @@ int sfmb200_estimate_e_mg(sfmb200_t* h, const int32_t* d_idx, int H_total, uint6
     CKL();
     h->mg_calls++;
     h->launches += 2;
-    h->have_candidates = false;        // the candidate arena holds this rank's slice only
+    h->st.lose_candidates();           // the candidate arena holds this rank's slice only
     return SFMB200_OK;
 }
 
@@ -770,86 +779,63 @@ int sfmb200_estimate_e_mg(sfmb200_t* h, const int32_t* d_idx, int H_total, uint6
 // far is accounted for.
 int sfmb200_mg_status(sfmb200_t* h, int32_t* h_timeouts) {
     ENTER(h);
-    if (!h || !h_timeouts) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !h_timeouts) return fail(SFMB200_ERR_ARG, "null argument");
     *h_timeouts = 0;
     if (!h->mg_failed_host) return SFMB200_OK;
     CK(cudaStreamSynchronize(h->stream));
     *h_timeouts = *(volatile int*)h->mg_failed_host;
-    if (*h_timeouts != 0) h->have_E = false;
+    if (*h_timeouts != 0) h->st.lose_essential();
     return SFMB200_OK;
 }
 
 int sfmb200_best_buffer(sfmb200_t* h, uint64_t** d_best) {
     ENTER(h);
-    if (!h || !d_best) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !d_best) return fail(SFMB200_ERR_ARG, "null argument");
     *d_best = (uint64_t*)h->s.best;
     return SFMB200_OK;
 }
 int sfmb200_adopt_best(sfmb200_t* h, const int32_t* d_idx, int H_total, uint64_t seed) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!h->have_points) return fail(SFMB200_ERR_STATE, "adopt_best before set_points%s");
-    if (h->model != 0 || !(h->thr > 0.0f))
-        return fail(SFMB200_ERR_STATE, "adopt_best follows an essential-matrix estimate (estimate_e / estimate_e_slice) on this handle%s");
+    ENTER_HANDLE(h);
+    if (int rc = need(h, NEED_POINTS, "adopt_best before set_points")) return rc;
+    if (h->st.E == Held::homography || !(h->thr > 0.0f))
+        return fail(SFMB200_ERR_STATE, "adopt_best follows an essential-matrix estimate (estimate_e / estimate_e_slice) on this handle");
     launch_regen_best(h->s, d_idx, (long long)H_total * 8, seed, h->hyp_solver, h->stream);
     CKL();
     h->launches++;
-    h->have_E = true;
-    h->have_pose = false;
-    h->have_chain = false;
-    h->model = 0;          // s.E is an essential matrix scored at h->thr (set by the slice estimate that preceded)
+    h->st.new_E();         // an essential matrix scored at h->thr (set by the slice estimate that preceded)
     return SFMB200_OK;
 }
 
 int sfmb200_refine_e(sfmb200_t* h, int iterations) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (iterations < 0 || iterations > 64) return fail(SFMB200_ERR_ARG, "iterations must be in [0, 64]%s");
-    if (!h->have_E || !h->have_points) return fail(SFMB200_ERR_STATE, "refine_e before an essential matrix exists%s");
+    ENTER_HANDLE(h);
+    if (iterations < 0 || iterations > 64) return fail(SFMB200_ERR_ARG, "iterations must be in [0, 64]");
+    if (int rc = need(h, NEED_POINTS | NEED_ESSENTIAL, "refine_e before an essential matrix exists")) return rc;
     if (iterations == 0) return SFMB200_OK;
-    h->launches += launch_refit(h->s, h->refit, h->thr > 0 ? h->thr : 1e-6f, iterations, h->stream);
+    h->launches += launch_refit(h->s, h->refit, stage_thr(h), iterations, h->stream);
     CKL();
-    h->have_pose = false;
-    h->have_chain = false;
+    h->st.new_E();
     return SFMB200_OK;
 }
 // Scratch of the bundle adjustment: allocated on first use so that handles that never adjust (the batched
 // configs: thousands of pairs) do not carry 25 bytes per correspondence for it.
 static int ensure_ba_arena(sfmb200_handle* h) {
-    if (h->ba_arena) return SFMB200_OK;
-    const DeviceState& s = h->s;
-    const size_t B = s.B;
-    int ba_blocks = (592 + s.B - 1) / s.B;          // LM kernels: ~4 CTAs per SM over the whole batch
-    ba_blocks = ba_blocks < 2 ? 2 : (ba_blocks > 296 ? 296 : ba_blocks);
-    size_t off = 0;
-    auto carve = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-    size_t o_bp = carve(B * 2 * 3 * (size_t)s.n_stride * sizeof(float));
-    size_t o_ba = carve(B * (size_t)s.n_stride);
-    size_t o_bc2 = carve(B * 24 * sizeof(float));
-    size_t o_bd = carve(B * 6 * sizeof(double));
-    size_t o_bi2 = carve(B * 8 * sizeof(int));
-    size_t o_bf = carve(B * 8 * sizeof(float));
-    size_t o_bpart = carve(B * ba_blocks * 34 * sizeof(double));
-    size_t o_bpart2 = carve(B * ba_blocks * 2 * sizeof(double));
-    size_t o_bs = carve(B * 8 * sizeof(float));
-    size_t o_bcand = carve(B * 32 * sizeof(float));
-    size_t o_bbase = carve(B * sizeof(int));
-    CK(cudaMalloc(&h->ba_arena, off));
-    CK(cudaMemsetAsync(h->ba_arena, 0, off, h->stream));
-    char* base = (char*)h->ba_arena;
-    h->ba.pts = (float*)(base + o_bp);
-    h->ba.active = (unsigned char*)(base + o_ba);
-    h->ba.cam = (float*)(base + o_bc2);
-    h->ba.dc = (double*)(base + o_bd);
-    h->ba.ctl_i = (int*)(base + o_bi2);
-    h->ba.ctl_f = (float*)(base + o_bf);
-    h->ba.part = (double*)(base + o_bpart);
-    h->ba.part2 = (double*)(base + o_bpart2);
-    h->ba.stats = (float*)(base + o_bs);
-    h->ba.cand = (float*)(base + o_bcand);
-    h->ba.base_count = (int*)(base + o_bbase);
-    h->ba.max_blocks = ba_blocks;
-    return SFMB200_OK;
+    const size_t B = h->s.B, n = h->s.n_stride;
+    BAState& ba = h->ba;
+    int ba_blocks = (592 + h->s.B - 1) / h->s.B;          // LM kernels: ~4 CTAs per SM over the whole batch
+    ba.max_blocks = ba_blocks < 2 ? 2 : (ba_blocks > 296 ? 296 : ba_blocks);
+    return lazy_arena(h, &h->ba_arena, [&](Carver& carve) {
+        carve(&ba.pts, B * 2 * 3 * n);
+        carve(&ba.active, B * n);
+        carve(&ba.cam, B * 24);
+        carve(&ba.dc, B * 6);
+        carve(&ba.ctl_i, B * 8);
+        carve(&ba.ctl_f, B * 8);
+        carve(&ba.part, B * ba.max_blocks * 34);
+        carve(&ba.part2, B * ba.max_blocks * 2);
+        carve(&ba.stats, B * 8);
+        carve(&ba.cand, B * 32);
+        carve(&ba.base_count, B);
+    });
 }
 
 // Bundle adjustment of the selected pose and the triangulated inliers with inlier re-selection
@@ -858,16 +844,14 @@ static int ensure_ba_arena(sfmb200_handle* h) {
 // [pairs][8]): active points, cost at entry, cost at exit, accepted steps, lambda, gauge scale,
 // inliers of the refined E, spare - of the LAST round.
 int sfmb200_bundle_adjust(sfmb200_t* h, int outer_rounds, int iterations, float* h_stats) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
+    ENTER_HANDLE(h);
     if (outer_rounds < 1 || outer_rounds > 64 || iterations < 1 || iterations > 256)
-        return fail(SFMB200_ERR_ARG, "outer_rounds in [1, 64] and iterations in [1, 256] required%s");
-    if (!h->have_points || !h->have_E || !h->have_pose || h->model != 0)
-        return fail(SFMB200_ERR_STATE, "bundle_adjust needs an essential matrix and a chosen pose%s");
-    const float thr = h->thr > 0 ? h->thr : 1e-6f;
+        return fail(SFMB200_ERR_ARG, "outer_rounds in [1, 64] and iterations in [1, 256] required");
+    if (int rc = need(h, NEED_POINTS | NEED_ESSENTIAL | NEED_POSE, "bundle_adjust needs an essential matrix and a chosen pose"))
+        return rc;
     if (int rc = ensure_ba_arena(h)) return rc;
     for (int r = 0; r < outer_rounds; r++) {
-        h->launches += launch_bundle_adjust(h->s, h->ba, thr, iterations, 1e-3f, h->tri_inliers_only, r == 0, h->ba.stats, h->stream);
+        h->launches += launch_bundle_adjust(h->s, h->ba, stage_thr(h), iterations, 1e-3f, h->tri_inliers_only, r == 0, h->ba.stats, h->stream);
         CKL();
     }
     if (h_stats) {
@@ -879,37 +863,31 @@ int sfmb200_bundle_adjust(sfmb200_t* h, int outer_rounds, int iterations, float*
 
 // N-view chaining (chain.cu): pairs of the handle = consecutive view pairs over index-aligned tracks.
 int sfmb200_chain_views(sfmb200_t* h, float* d_cloud, int32_t* d_count, float* h_cameras, float* h_scales, int32_t* h_used) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (h->s.B > 256) return fail(SFMB200_ERR_ARG, "chain_views handles at most 256 pairs (257 views)%s");
-    if (!h->have_points || !h->have_E || !h->have_pose || h->model != 0)
-        return fail(SFMB200_ERR_STATE, "chain_views needs an essential matrix, a chosen pose and triangulated points per pair%s");
+    ENTER_HANDLE(h);
+    if (h->s.B > 256) return fail(SFMB200_ERR_ARG, "chain_views handles at most 256 pairs (257 views)");
+    if (int rc = need(h, NEED_POINTS | NEED_ESSENTIAL | NEED_POSE,
+                      "chain_views needs an essential matrix, a chosen pose and triangulated points per pair"))
+        return rc;
     const size_t B = h->s.B;
-    if (!h->chain_arena) {
-        size_t off = 0;
-        auto carve = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-        size_t o_h = carve(B * 2048 * sizeof(int)), o_m = carve(B * sizeof(int)), o_u = carve(B * sizeof(int));
-        size_t o_s = carve(B * sizeof(unsigned long long)), o_c = carve(B * sizeof(int)), o_sc = carve(B * sizeof(float));
-        size_t o_cs = carve(B * sizeof(float)), o_cam = carve((B + 1) * 12 * sizeof(float));
-        CK(cudaMalloc(&h->chain_arena, off));
-        char* base = (char*)h->chain_arena;
-        h->chain.hist = (int*)(base + o_h);
-        h->chain.median_bin = (int*)(base + o_m);
-        h->chain.used = (int*)(base + o_u);
-        h->chain.bin_sum = (unsigned long long*)(base + o_s);
-        h->chain.bin_cnt = (int*)(base + o_c);
-        h->chain.scales = (float*)(base + o_sc);
-        h->chain.cum_scales = (float*)(base + o_cs);
-        h->chain.cameras = (float*)(base + o_cam);
-        CK(cudaMemsetAsync(h->chain_arena, 0, off, h->stream));
-    }
-    h->launches += launch_chain(h->s, h->chain, h->thr > 0 ? h->thr : 1e-6f, d_cloud, d_count, h->stream);
+    ChainState& c = h->chain;
+    int rc = lazy_arena(h, &h->chain_arena, [&](Carver& carve) {
+        carve(&c.hist, B * 2048);
+        carve(&c.median_bin, B);
+        carve(&c.used, B);
+        carve(&c.bin_sum, B);
+        carve(&c.bin_cnt, B);
+        carve(&c.scales, B);
+        carve(&c.cum_scales, B);
+        carve(&c.cameras, (B + 1) * 12);
+    });
+    if (rc) return rc;
+    h->launches += launch_chain(h->s, c, stage_thr(h), d_cloud, d_count, h->stream);
     CKL();
-    if (h_cameras) CK(cudaMemcpyAsync(h_cameras, h->chain.cameras, (B + 1) * 12 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    if (h_scales) CK(cudaMemcpyAsync(h_scales, h->chain.scales, B * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    if (h_used) CK(cudaMemcpyAsync(h_used, h->chain.used, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    if (h_cameras) CK(cudaMemcpyAsync(h_cameras, c.cameras, (B + 1) * 12 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    if (h_scales) CK(cudaMemcpyAsync(h_scales, c.scales, B * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    if (h_used) CK(cudaMemcpyAsync(h_used, c.used, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     if (h_cameras || h_scales || h_used) CK(cudaStreamSynchronize(h->stream));
-    h->have_chain = true;
+    h->st.chained();
     return SFMB200_OK;
 }
 
@@ -917,80 +895,67 @@ int sfmb200_chain_views(sfmb200_t* h, float* d_cloud, int32_t* d_count, float* h
 int sfmb200_bundle_adjust_global(sfmb200_t* h, float* d_cloud, const int32_t* d_count, int iterations, float* h_cameras,
                                  float* h_stats) {
     ENTER(h);
-    if (!h || !d_cloud || !d_count) return fail(SFMB200_ERR_ARG, "null argument%s");
-    if (iterations < 1 || iterations > 1000) return fail(SFMB200_ERR_ARG, "iterations must be in [1, 1000]%s");
-    if (h->s.B > GBA_MAX_PAIRS) return fail(SFMB200_ERR_ARG, "bundle_adjust_global handles at most 16 pairs (17 views)%s");
-    if (!h->have_chain || !h->chain_arena || !h->have_points || !h->have_E || !h->have_pose || h->model != 0)
-        return fail(SFMB200_ERR_STATE, "bundle_adjust_global follows chain_views (cloud and count from that call)%s");
-    const DeviceState& s = h->s;
-    if (!h->gba_arena) {
-        const size_t V = s.B + 1, n = s.n_max;
-        const int nb = 148;
-        size_t off = 0;
-        auto carve = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-        size_t o_cam = carve(2 * V * 12 * sizeof(float)), o_pts = carve(2 * 3 * n * sizeof(float)), o_obs = carve(n * sizeof(unsigned int));
-        size_t o_lin = carve(n * 9 * sizeof(float)), o_part = carve(gba_part_doubles(s.B, nb) * sizeof(double));
-        size_t o_p2 = carve((size_t)nb * 2 * sizeof(double)), o_dc = carve(6 * (size_t)s.B * sizeof(double));
-        size_t o_ci = carve(8 * sizeof(int)), o_cf = carve(8 * sizeof(float)), o_st = carve(8 * sizeof(float));
-        CK(cudaMalloc(&h->gba_arena, off));
-        CK(cudaMemsetAsync(h->gba_arena, 0, off, h->stream));
-        char* base = (char*)h->gba_arena;
-        h->gba.cam = (float*)(base + o_cam);
-        h->gba.pts = (float*)(base + o_pts);
-        h->gba.obs = (unsigned int*)(base + o_obs);
-        h->gba.lin = (float*)(base + o_lin);
-        h->gba.part = (double*)(base + o_part);
-        h->gba.part2 = (double*)(base + o_p2);
-        h->gba.dc = (double*)(base + o_dc);
-        h->gba.ctl_i = (int*)(base + o_ci);
-        h->gba.ctl_f = (float*)(base + o_cf);
-        h->gba.nb = nb;
-        h->gba_stats = (float*)(base + o_st);
-    }
-    float* d_stats = h->gba_stats;
-    h->launches += launch_global_ba(h->s, h->chain, h->gba, h->thr > 0 ? h->thr : 1e-6f, iterations, d_cloud, d_count, d_stats, h->stream);
+    if (!h || !d_cloud || !d_count) return fail(SFMB200_ERR_ARG, "null argument");
+    if (iterations < 1 || iterations > 1000) return fail(SFMB200_ERR_ARG, "iterations must be in [1, 1000]");
+    if (h->s.B > GBA_MAX_PAIRS) return fail(SFMB200_ERR_ARG, "bundle_adjust_global handles at most 16 pairs (17 views)");
+    if (int rc = need(h, NEED_CHAIN | NEED_POINTS | NEED_ESSENTIAL | NEED_POSE,
+                      "bundle_adjust_global follows chain_views (cloud and count from that call)"))
+        return rc;
+    const size_t B = h->s.B, V = B + 1, n = h->s.n_max;
+    GbaState& g = h->gba;
+    g.nb = 148;
+    int rc = lazy_arena(h, &h->gba_arena, [&](Carver& carve) {
+        carve(&g.cam, 2 * V * 12);
+        carve(&g.pts, 2 * 3 * n);
+        carve(&g.obs, n);
+        carve(&g.lin, n * 9);
+        carve(&g.part, gba_part_doubles(h->s.B, g.nb));
+        carve(&g.part2, (size_t)g.nb * 2);
+        carve(&g.dc, 6 * B);
+        carve(&g.ctl_i, 8);
+        carve(&g.ctl_f, 8);
+        carve(&h->gba_stats, 8);
+    });
+    if (rc) return rc;
+    h->launches += launch_global_ba(h->s, h->chain, g, stage_thr(h), iterations, d_cloud, d_count, h->gba_stats, h->stream);
     CKL();
-    const size_t B = h->s.B;
-    if (h_cameras) CK(cudaMemcpyAsync(h_cameras, h->chain.cameras, (B + 1) * 12 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    if (h_stats) CK(cudaMemcpyAsync(h_stats, d_stats, 8 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    if (h_cameras) CK(cudaMemcpyAsync(h_cameras, h->chain.cameras, V * 12 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    if (h_stats) CK(cudaMemcpyAsync(h_stats, h->gba_stats, 8 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     if (h_cameras || h_stats) CK(cudaStreamSynchronize(h->stream));
     return SFMB200_OK;
 }
 
 int sfmb200_get_refit_iterations(sfmb200_t* h, int32_t* h_iters) {
     ENTER(h);
-    if (!h || !h_iters) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !h_iters) return fail(SFMB200_ERR_ARG, "null argument");
     CK(cudaMemcpyAsync(h_iters, h->refit.iters_done, (size_t)h->s.B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return SFMB200_OK;
 }
 
 int sfmb200_pose_candidates(sfmb200_t* h) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!h->have_E) return fail(SFMB200_ERR_STATE, "pose_candidates before an essential matrix exists%s");
+    ENTER_HANDLE(h);
+    if (int rc = need(h, NEED_ESSENTIAL, "pose_candidates before an essential matrix exists")) return rc;
     launch_pose_candidates(h->s, h->compat, h->stream);
     prof_mark(h, 5);
     CKL();
     h->launches++;
-    h->have_pose = true;
+    h->st.poses();
     return SFMB200_OK;
 }
 int sfmb200_choose_pose(sfmb200_t* h) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!h->have_pose || !h->have_points) return fail(SFMB200_ERR_STATE, "choose_pose before pose_candidates%s");
-    launch_choose_pose(h->s, h->compat, h->thr > 0 ? h->thr : 1e-6f, h->stream);
+    ENTER_HANDLE(h);
+    if (int rc = need(h, NEED_POSE | NEED_POINTS, "choose_pose before pose_candidates")) return rc;
+    launch_choose_pose(h->s, h->compat, stage_thr(h), h->stream);
     prof_mark(h, 6);
     CKL();
     h->launches++;
     return SFMB200_OK;
 }
 int sfmb200_triangulate(sfmb200_t* h) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!h->have_pose || !h->have_points) return fail(SFMB200_ERR_STATE, "triangulate before pose_candidates%s");
-    launch_triangulate(h->s, h->tri_inliers_only, h->thr > 0 ? h->thr : 1e-6f, h->stream);
+    ENTER_HANDLE(h);
+    if (int rc = need(h, NEED_POSE | NEED_POINTS, "triangulate before pose_candidates")) return rc;
+    launch_triangulate(h->s, h->tri_inliers_only, stage_thr(h), h->stream);
     prof_mark(h, 7);
     CKL();
     h->launches++;
@@ -1001,56 +966,17 @@ int sfmb200_triangulate(sfmb200_t* h) {
 // select + pose candidates + cheirality kernel, [inlier vote in non-compat mode],
 // triangulation.  Stage marks 4..6 collapse onto the fused kernel.
 static int run_stages(sfmb200_t* h, int H, uint64_t seed, float thr) {
-    if (!h->have_points) return fail(SFMB200_ERR_STATE, "run before set_points%s");
-    if (H < 1 || H > h->s.h_max) return fail(SFMB200_ERR_ARG, "H out of range / above max_hypotheses%s");
-    if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive%s");
     h->H = H;
     h->h_begin = 0;
     h->thr = thr;
     if (int rc = ensure_scaled(h, make_thr_scale(thr).ik)) return rc;     // no-op after run_device / run_host's own ingest
     h->plan = plan_essential(h, h->s.n, H);
-    int chunks = h->pipeline_chunks;
-    if (chunks < 0) chunks = 1;      // measured on B200 (profiles/r02_batch_pipeline.md): no gain at config 4, so off unless asked for
-    if (chunks > h->s.B) chunks = h->s.B;
-    if (chunks >= 2) {
-        // Batched pipeline: the batch is cut into chunks of pairs; hypothesis generation of ALL chunks is enqueued on a
-        // side stream, scoring of chunk c on the main stream waits only for generation of chunk c.  The persistent
-        // scoring grid holds one 256-thread CTA (42 K registers) per SM, which leaves room for one 128-thread generation
-        // CTA next to it: generation - a latency-bound kernel that keeps the FMA pipe 40 % busy on its own - runs in the
-        // issue slots scoring leaves idle instead of in front of it.  Same kernels, same per-pair seeds: same bits.
-        if (!h->aux_stream) {
-            CK(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
-            CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-            for (int i = 0; i < 16; i++) CK(cudaEventCreateWithFlags(&h->ev_chunk[i], cudaEventDisableTiming));
-        }
-        CK(cudaEventRecord(h->ev_fork, h->stream));
-        CK(cudaStreamWaitEvent(h->aux_stream, h->ev_fork, 0));
-        const int per = (h->s.B + chunks - 1) / chunks;
-        int used = 0;
-        for (int c = 0, b0 = 0; b0 < h->s.B; c++, b0 += per, used++) {
-            const DeviceState v = sub_batch(h->s, b0, b0 + per <= h->s.B ? per : h->s.B - b0);
-            launch_hypgen(v, nullptr, (long long)H * 8, H, 0, seed, h->hyp_solver, h->aux_stream);
-            CKL();
-            CK(cudaEventRecord(h->ev_chunk[c], h->aux_stream));
-        }
-        for (int c = 0, b0 = 0; b0 < h->s.B; c++, b0 += per) {
-            const DeviceState v = sub_batch(h->s, b0, b0 + per <= h->s.B ? per : h->s.B - b0);
-            CK(cudaStreamWaitEvent(h->stream, h->ev_chunk[c], 0));
-            ScorePlan keep = h->plan;
-            h->plan = h->s.metric == 0 ? make_score_plan(v.B, v.n, H, h->score_variant, h->sms) : make_score_plan_homography(v.B, v.n, H, h->sms);
-            score_essential(h, v, H, 0, thr);
-            CKL();
-            h->plan = keep;
-        }
-        h->launches += 2 * used - 2;
-    } else {
-        launch_hypgen(h->s, nullptr, (long long)H * 8, H, 0, seed, h->hyp_solver, h->stream);
-        prof_mark(h, 2);
-        CKL();
-        score_essential(h, h->s, H, 0, thr);
-        prof_mark(h, 3);
-        CKL();
-    }
+    launch_hypgen(h->s, nullptr, (long long)H * 8, H, 0, seed, h->hyp_solver, h->stream);
+    prof_mark(h, 2);
+    CKL();
+    score_essential(h, h->s, H, 0, thr);
+    prof_mark(h, 3);
+    CKL();
     launch_select_pose_choose(h->s, 0, h->compat, h->stream);
     prof_mark(h, 4);
     prof_mark(h, 5);
@@ -1062,47 +988,53 @@ static int run_stages(sfmb200_t* h, int H, uint64_t seed, float thr) {
         h->launches++;
     }
     prof_mark(h, 6);
-    h->have_candidates = h->have_E = h->have_pose = true;
-    h->have_chain = false;        // a new reconstruction: what chain_views left is stale
-    h->model = 0;                 // s.E is an essential matrix again (find_homography may have run on this handle before)
+    h->st.estimate(Held::essential);
+    h->st.poses();
     return sfmb200_triangulate(h);
 }
 
-// Whole path in ONE launch when the problem is small (small.cu).  Returns 0 when the fused path does not apply (the
-// caller continues with the general path), 1 when it ran, < 0 on error.  d_px: device-readable pixel correspondences.
+// Whole path in ONE launch (small.cu), for the problems small_path_ok admits.  d_px: device-readable pixel
+// correspondences.
 static int run_small(sfmb200_t* h, const float* d_px, int n, int H, uint64_t seed, float thr) {
-    if (!d_px || n < 8 || n > h->s.n_max || H < 1 || H > h->s.h_max) return 0;       // let the general path report the error
-    const int n_before = h->s.n;
-    h->s.n = n;
-    const bool ok = small_path_ok(h, H, true);
-    h->s.n = n_before;
-    if (!ok) return 0;
     h->s.n = n;
     h->s.pt_scale = make_thr_scale(thr).ik;
     cudaError_t e = launch_small_path(h->s, d_px, nullptr, (long long)H * 8, H, 0, seed, thr, h->compat, h->tri_inliers_only,
                                       SMALL_INGEST | SMALL_ESTIMATE | SMALL_POSE | SMALL_TRI, h->stream);
-    if (e != cudaSuccess) return fail(SFMB200_ERR_CUDA, "fused small-problem launch: %s", cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail_cuda("fused small-problem launch", e);
     h->H = H;
     h->h_begin = 0;
     h->thr = thr;
-    h->model = 0;
     memset(&h->plan, 0, sizeof(h->plan));
     h->plan.variant = -2;
     h->launches += 1;
-    h->have_points = h->have_candidates = h->have_E = h->have_pose = true;
-    h->have_chain = false;
-    return 1;
+    h->st.new_points();
+    h->st.estimate(Held::essential);
+    h->st.poses();
+    return SFMB200_OK;
+}
+
+// Arguments of run_device / run_host.  All are checked before anything is enqueued, so a call that fails here leaves
+// the handle as it was.
+static int check_run(sfmb200_t* h, const void* px, int n, int H, float thr) {
+    if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive");
+    if (int rc = check_n(h, px, n)) return rc;
+    if (H < 1 || H > h->s.h_max) return fail(SFMB200_ERR_ARG, "H out of range / above max_hypotheses");
+    return SFMB200_OK;
+}
+
+// The whole path on validated arguments and device-readable pixel correspondences: the fused single launch when the
+// problem is small, else the ingest followed by the five-launch path.
+static int run_path(sfmb200_t* h, const float* d_px, int n, int H, uint64_t seed, float thr) {
+    if (small_path_ok(h, n, H, true)) return run_small(h, d_px, n, H, seed, thr);
+    if (int rc = ingest_xy(h, d_px, n, make_thr_scale(thr).ik)) return rc;     // writes the scaled copies for this threshold
+    return run_stages(h, H, seed, thr);
 }
 
 int sfmb200_run_device(sfmb200_t* h, const float* d_px, int n, int H, uint64_t seed, float thr) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive%s");
+    ENTER_HANDLE(h);
+    if (int rc = check_run(h, d_px, n, H, thr)) return rc;
     prof_next(h);
-    if (int rc = run_small(h, d_px, n, H, seed, thr)) return rc < 0 ? rc : SFMB200_OK;      // > 0: done by the fused path
-    int rc = ingest_xy(h, d_px, n, make_thr_scale(thr).ik);          // writes the scaled copies for this threshold
-    if (rc) return rc;
-    return run_stages(h, H, seed, thr);
+    return run_path(h, d_px, n, H, seed, thr);
 }
 
 // Results of the whole path packed for the host: one small header per pair and a
@@ -1144,41 +1076,23 @@ static void* pinned_alias(const void* host) {
 
 int sfmb200_run_host(sfmb200_t* h, const float* h_px, int n, int H, uint64_t seed, float thr, float* h_E, float* h_P,
                      int32_t* h_pose_index, int32_t* h_inliers, float* h_points) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
-    if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive%s");
+    ENTER_HANDLE(h);
+    if (int rc = check_run(h, h_px, n, H, thr)) return rc;
     prof_next(h);
-    const float scale = make_thr_scale(thr).ik;
     // zero copy pays where latency dominates (config-2-sized calls: 160 KB each way); bulk transfers (batched
     // config 4: hundreds of MB) stay with the copy engines, which keep more PCIe requests in flight than a kernel
     const size_t zero_copy_limit = 4u << 20;
-    const size_t in_bytes = (size_t)h->s.B * (size_t)(n > 0 ? n : 0) * 4 * sizeof(float);
-    const float* px_alias = in_bytes <= zero_copy_limit ? (const float*)pinned_alias(h_px) : nullptr;
-    int rc = 0;
-    const bool small_shape = h_px && n >= 8 && n <= h->s.n_max && H >= 1 && H <= h->s.h_max;
-    if (px_alias) {
-        rc = run_small(h, px_alias, n, H, seed, thr);
-    } else if (small_shape) {
-        // pageable input: stage it, then the fused path reads the staged copy
-        if ((rc = ensure_staging(h, true, false))) return rc;
-        CK(cudaMemcpyAsync(h->s.px, h_px, (size_t)h->s.B * n * 4 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-        rc = run_small(h, h->s.px, n, H, seed, thr);
-        if (rc == 0) {                                          // not eligible: general path on the staged copy
-            if ((rc = ingest_xy(h, h->s.px, n, scale))) return rc;
-            if ((rc = run_stages(h, H, seed, thr))) return rc;
-            rc = 1;
-        }
+    const size_t in_bytes = (size_t)h->s.B * n * 4 * sizeof(float);
+    const float* d_px = in_bytes <= zero_copy_limit ? (const float*)pinned_alias(h_px) : nullptr;
+    if (!d_px) {          // pageable, or too large for zero copy: one copy into the staging buffer
+        if (int rc = stage_input(h, h_px, n)) return rc;
+        d_px = h->px_staging;
     }
-    if (rc < 0) return rc;
-    if (rc == 0) {
-        rc = px_alias ? ingest_xy(h, px_alias, n, scale) : ingest_xy_host(h, h_px, n, scale);
-        if (rc) return rc;
-        if ((rc = run_stages(h, H, seed, thr))) return rc;
-    }
+    if (int rc = run_path(h, d_px, n, H, seed, thr)) return rc;
     DeviceState& s = h->s;
     const size_t B = s.B;
     float* pts_alias = B * 4 * (size_t)s.n * sizeof(float) <= zero_copy_limit ? (float*)pinned_alias(h_points) : nullptr;
-    if (h_points && !pts_alias && (rc = ensure_staging(h, false, true))) return rc;
+    if (h_points && !pts_alias && !h->pack_points) CK(cudaMalloc(&h->pack_points, B * 4 * (size_t)s.n_max * sizeof(float)));
     dim3 grid(h_points ? (s.n + 255) / 256 : 1, (unsigned)B);
     // header: always through the handle's own pinned buffer (device-visible under UVA); points: straight into the
     // caller's buffer when it is pinned, else into the device staging copy followed by one DMA
@@ -1200,7 +1114,7 @@ int sfmb200_run_host(sfmb200_t* h, const float* h_px, int n, int H, uint64_t see
 
 int sfmb200_copy_to_vbo(sfmb200_t* h, int pair, float* d_pos, float* d_col) {
     ENTER(h);
-    if (!h || pair < 0 || pair >= h->s.B) return fail(SFMB200_ERR_ARG, "bad handle / pair%s");
+    if (!h || pair < 0 || pair >= h->s.B) return fail(SFMB200_ERR_ARG, "bad handle / pair");
     launch_vbo(h->s, pair, d_pos, d_col, 1.0f, h->stream);
     CKL();
     h->launches++;
@@ -1210,10 +1124,12 @@ int sfmb200_copy_to_vbo(sfmb200_t* h, int pair, float* d_pos, float* d_col) {
 
 int sfmb200_copy_to_vbo_coloured(sfmb200_t* h, int pair, float* d_pos, float* d_col, float scale, int mode, float z_near, float z_far) {
     ENTER(h);
-    if (!h || pair < 0 || pair >= h->s.B) return fail(SFMB200_ERR_ARG, "bad handle / pair%s");
-    if (mode < 0 || mode > 2) return fail(SFMB200_ERR_ARG, "colour mode must be 0 (ones), 1 (inlier / outlier) or 2 (depth ramp)%s");
-    if (mode == 1 && (!h->have_E || h->model != 0)) return fail(SFMB200_ERR_STATE, "inlier colouring needs an essential matrix%s");
-    launch_vbo_colour(h->s, pair, d_pos, d_col, scale, mode, h->thr > 0 ? h->thr : 1e-6f, z_near, z_far, h->stream);
+    if (!h || pair < 0 || pair >= h->s.B) return fail(SFMB200_ERR_ARG, "bad handle / pair");
+    if (mode < 0 || mode > 2) return fail(SFMB200_ERR_ARG, "colour mode must be 0 (ones), 1 (inlier / outlier) or 2 (depth ramp)");
+    if (mode == 1) {
+        if (int rc = need(h, NEED_ESSENTIAL, "inlier colouring needs an essential matrix")) return rc;
+    }
+    launch_vbo_colour(h->s, pair, d_pos, d_col, scale, mode, stage_thr(h), z_near, z_far, h->stream);
     CKL();
     h->launches++;
     CK(cudaStreamSynchronize(h->stream));
@@ -1222,26 +1138,23 @@ int sfmb200_copy_to_vbo_coloured(sfmb200_t* h, int pair, float* d_pos, float* d_
 
 int sfmb200_get_E(sfmb200_t* h, float* h_E) {
     ENTER(h);
-    if (!h || !h_E) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !h_E) return fail(SFMB200_ERR_ARG, "null argument");
     CK(cudaMemcpyAsync(h_E, h->s.E, (size_t)h->s.B * 9 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return SFMB200_OK;
 }
 int sfmb200_set_E(sfmb200_t* h, const float* h_E) {
     ENTER(h);
-    if (!h || !h_E) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !h_E) return fail(SFMB200_ERR_ARG, "null argument");
     CK(cudaMemcpyAsync(h->s.E, h_E, (size_t)h->s.B * 9 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    h->have_E = true;
-    h->have_pose = false;
-    h->have_chain = false;
-    h->model = 0;
+    h->st.new_E();
     if (!(h->thr > 0)) h->thr = 1e-6f;
     return SFMB200_OK;
 }
 int sfmb200_get_best(sfmb200_t* h, int32_t* h_index, int32_t* h_count) {
     ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h) return fail(SFMB200_ERR_ARG, "null argument");
     if (h_index) CK(cudaMemcpyAsync(h_index, h->s.best_idx, (size_t)h->s.B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     if (h_count) CK(cudaMemcpyAsync(h_count, h->s.best_count, (size_t)h->s.B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -1249,21 +1162,21 @@ int sfmb200_get_best(sfmb200_t* h, int32_t* h_index, int32_t* h_count) {
 }
 int sfmb200_get_poses(sfmb200_t* h, float* h_P) {
     ENTER(h);
-    if (!h || !h_P) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !h_P) return fail(SFMB200_ERR_ARG, "null argument");
     CK(cudaMemcpyAsync(h_P, h->s.P, (size_t)h->s.B * 64 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return SFMB200_OK;
 }
 int sfmb200_get_pose_index(sfmb200_t* h, int32_t* h_ind) {
     ENTER(h);
-    if (!h || !h_ind) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !h_ind) return fail(SFMB200_ERR_ARG, "null argument");
     CK(cudaMemcpyAsync(h_ind, h->s.P_ind, (size_t)h->s.B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return SFMB200_OK;
 }
 static int check_pair(sfmb200_t* h, int pair, const void* p) {
-    if (!h || !p) return fail(SFMB200_ERR_ARG, "null argument%s");
-    if (pair < 0 || pair >= h->s.B) return fail(SFMB200_ERR_ARG, "pair out of range%s");
+    if (!h || !p) return fail(SFMB200_ERR_ARG, "null argument");
+    if (pair < 0 || pair >= h->s.B) return fail(SFMB200_ERR_ARG, "pair out of range");
     return SFMB200_OK;
 }
 int sfmb200_get_points(sfmb200_t* h, int pair, float* d_points) {
@@ -1291,7 +1204,7 @@ int sfmb200_get_inlier_counts(sfmb200_t* h, int pair, int32_t* d_counts) {
     ENTER(h);
     int rc = check_pair(h, pair, d_counts);
     if (rc) return rc;
-    if (!h->have_candidates) return fail(SFMB200_ERR_STATE, "no estimate yet%s");
+    if ((rc = need(h, NEED_CANDIDATES, "no estimate yet"))) return rc;
     CK(cudaMemcpyAsync(d_counts, h->s.counts + (size_t)pair * h->s.h_stride, (size_t)h->H * sizeof(int),
                        cudaMemcpyDeviceToDevice, h->stream));
     return SFMB200_OK;
@@ -1300,7 +1213,7 @@ int sfmb200_get_E_candidates(sfmb200_t* h, int pair, float* d_E) {
     ENTER(h);
     int rc = check_pair(h, pair, d_E);
     if (rc) return rc;
-    if (!h->have_candidates) return fail(SFMB200_ERR_STATE, "no estimate yet%s");
+    if ((rc = need(h, NEED_CANDIDATES, "no estimate yet"))) return rc;
     launch_export_ecand(h->s, pair, h->H, d_E, h->stream);
     CKL();
     h->launches++;
@@ -1310,8 +1223,8 @@ int sfmb200_get_X(sfmb200_t* h, int pair, int image, float* d_X) {
     ENTER(h);
     int rc = check_pair(h, pair, d_X);
     if (rc) return rc;
-    if (image < 0 || image > 1) return fail(SFMB200_ERR_ARG, "image must be 0 or 1%s");
-    if (!h->have_points) return fail(SFMB200_ERR_STATE, "no points yet%s");
+    if (image < 0 || image > 1) return fail(SFMB200_ERR_ARG, "image must be 0 or 1");
+    if ((rc = need(h, NEED_POINTS, "no points yet"))) return rc;
     launch_export_X(h->s, pair, image, d_X, h->stream);
     CKL();
     h->launches++;
@@ -1321,16 +1234,15 @@ int sfmb200_get_inlier_mask(sfmb200_t* h, int pair, uint8_t* d_mask) {
     ENTER(h);
     int rc = check_pair(h, pair, d_mask);
     if (rc) return rc;
-    if (!(h->have_E || h->model == 1) || !h->have_points) return fail(SFMB200_ERR_STATE, "no model yet%s");
-    launch_inlier_mask(h->s, pair, h->thr > 0 ? h->thr : 1e-6f, h->model, d_mask, h->stream);
+    if ((rc = need(h, NEED_MODEL | NEED_POINTS, "no model yet"))) return rc;
+    launch_inlier_mask(h->s, pair, stage_thr(h), h->st.E == Held::homography ? 1 : 0, d_mask, h->stream);
     CKL();
     h->launches++;
     return SFMB200_OK;
 }
 int sfmb200_device_views(sfmb200_t* h, float** d_E, float** d_P, int32_t** d_pose_index, float** d_points,
                          int* point_stride) {
-    ENTER(h);
-    if (!h) return fail(SFMB200_ERR_ARG, "null handle%s");
+    ENTER_HANDLE(h);
     if (d_E) *d_E = h->s.E;
     if (d_P) *d_P = h->s.P;
     if (d_pose_index) *d_pose_index = h->s.P_ind;
@@ -1340,7 +1252,7 @@ int sfmb200_device_views(sfmb200_t* h, float** d_E, float** d_P, int32_t** d_pos
 }
 int sfmb200_score_plan(sfmb200_t* h, int32_t out[4]) {
     ENTER(h);
-    if (!h || !out) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !out) return fail(SFMB200_ERR_ARG, "null argument");
     out[0] = h->plan.variant;
     out[1] = h->plan.tiles;
     out[2] = h->plan.ctas;
@@ -1351,9 +1263,9 @@ int64_t sfmb200_launch_count(sfmb200_t* h) { return h ? h->launches : 0; }
 
 int sfmb200_stage_times(sfmb200_t* h, int max_sets, float* ms, int* sets) {
     ENTER(h);
-    if (!h || !ms || !sets) return fail(SFMB200_ERR_ARG, "null argument%s");
+    if (!h || !ms || !sets) return fail(SFMB200_ERR_ARG, "null argument");
     *sets = 0;
-    if (!h->prof_ev) return fail(SFMB200_ERR_STATE, "profiling was never enabled%s");
+    if (!h->prof_ev) return fail(SFMB200_ERR_STATE, "profiling was never enabled");
     CK(cudaStreamSynchronize(h->stream));
     long long have = h->prof_total < PROF_RING ? h->prof_total : PROF_RING;
     long long first = h->prof_total - have;
@@ -1372,7 +1284,7 @@ int sfmb200_small_path_debug(int64_t* d_stamps) {
 }
 
 int sfmb200_fma_probe(int mode, int iters, double* fmas, float* ms) {
-    if (!fmas || !ms || iters < 1 || mode < 0 || mode > 4) return fail(SFMB200_ERR_ARG, "bad argument%s");
+    if (!fmas || !ms || iters < 1 || mode < 0 || mode > 4) return fail(SFMB200_ERR_ARG, "bad argument");
     float* sink = nullptr;
     cudaEvent_t e0, e1;
     CK(cudaMalloc(&sink, 256));

@@ -24,9 +24,13 @@ constexpr int SCORE_MIN_TILE = 256;  // smallest hypothesis tile of any kernel v
 
 // Everything one handle owns on the device.  All per-pair arrays are laid out
 // [pair][...] with fixed strides so a batch is one launch (blockIdx.y / z = pair).
+// The struct is every kernel's first parameter, and the code nvcc schedules for the scoring kernels depends on where
+// the fields sit in it: moving corr .. vote by 8 bytes made the flagship step 1.3 % slower (B200, 1000 W power
+// limit).  Add fields at the end.
 struct DeviceState {
     int B;              // pairs in the batch
-    int pair0;          // index of this view's first pair in the handle's batch (sub-batch launches; seeds the per-pair sampler)
+    int sampler;        // device-drawn sample rows: 0 independent 8-subsets per hypothesis, 1 one permutation cut into disjoint
+                        // groups of 8 (the reference's scheme, sfm.cu:95-104)
     int n_max;          // capacity: correspondences per pair
     int h_max;          // capacity: hypotheses per pair (local slice)
     int n;              // current correspondences per pair
@@ -39,7 +43,8 @@ struct DeviceState {
     float pt_scale;     // 1/sqrt(thr) currently materialised in corr_s (sampson.cuh); 1 for the homography model
     float4* corr;       // [B][n_stride]   (x1,y1,x2,y2) normalised camera coords
     float4* corr_s;     // [B][n_stride]   corr * pt_scale: what the scalar scoring kernels stage
-    float* px;          // [B][n_stride][4] staging for host pixel input (device)
+    const int* skip;    // adaptive termination: when non-null and *skip != 0 the hypgen / score kernels of
+                        // the remaining rounds return at once (set by adaptive_decide_kernel); else nullptr
     float* Ecand;       // [B][9][h_stride] SoA essential-matrix candidates
     int* counts;        // [B][h_stride] inlier count per hypothesis
     int* tile_done;     // [B][tiles_max] split tickets per hypothesis tile
@@ -52,36 +57,8 @@ struct DeviceState {
     float* points;      // [B][4][n_stride] SoA (x,y,z,1), the reference's d_final_points layout
     int* tri_count;     // [B] points triangulated in front of both cameras (diagnostic)
     int* vote;          // [B][8] cheirality votes of the four candidates + ticket (choose_pose_vote_kernel)
-    int sampler;        // device-drawn sample rows: 0 independent 8-subsets per hypothesis, 1 one permutation cut into disjoint
-                        // groups of 8 (the reference's scheme, sfm.cu:95-104)
     int metric;         // inlier test of the essential-matrix model: 0 Sampson error (default), 1 symmetric epipolar distance
-    const int* skip;    // adaptive termination: when non-null and *skip != 0 the hypgen / score kernels of
-                        // the remaining rounds return at once (set by adaptive_decide_kernel); else nullptr
 };
-
-// A view of pairs [b0, b0 + nb) of the batch: every per-pair array advanced to pair b0, B = nb.  Kernels that derive
-// anything from the pair's absolute index (the sampler seed) use pair0 + blockIdx.y.
-inline DeviceState sub_batch(const DeviceState& s, int b0, int nb) {
-    DeviceState v = s;
-    const size_t b = (size_t)b0;
-    v.B = nb;
-    v.pair0 = s.pair0 + b0;
-    v.corr += b * s.n_stride;
-    v.corr_s += b * s.n_stride;
-    v.Ecand += b * 9 * s.h_stride;
-    v.counts += b * s.h_stride;
-    v.tile_done += b * s.tiles_max;
-    v.best += b;
-    v.E += b * 9;
-    v.best_idx += b;
-    v.best_count += b;
-    v.P += b * 64;
-    v.P_ind += b;
-    v.points += b * 4 * s.n_stride;
-    v.tri_count += b;
-    v.vote += b * 8;
-    return v;
-}
 
 // Scratch of the local-optimisation (refit) stage, per pair.
 struct RefitState {

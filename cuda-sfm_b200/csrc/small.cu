@@ -98,7 +98,7 @@ __global__ void __launch_bounds__(SMALL_THREADS, 1) small_path_kernel(DeviceStat
             const bool live = j < H;
             Corr pts[8];
             float E[9];
-            const bool ok = load_sample<true>(corr, n, rows, a.seed + 0x632BE59BD9B4E019ull * (unsigned long long)(s.pair0 + b),
+            const bool ok = load_sample<true>(corr, n, rows, a.seed + 0x632BE59BD9B4E019ull * (unsigned long long)b,
                                               (long long)a.h_offset + (live ? j : 0), pts, s.sampler);
             solve_hypothesis_projector(pts, E);
             if (live) {

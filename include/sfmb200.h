@@ -62,10 +62,6 @@ typedef enum {
                                       SFMB200_OPT_SMALL_PATH_EVALS, 0 never, 1 whenever eligible (projector solver,
                                       H <= 128 * cluster size, reference pose semantics, no per-stage profiling) */
     SFMB200_OPT_SMALL_PATH_EVALS = 8, /* the n * H limit of the automatic choice (default 2,500,000; the automatic choice also needs <= 4 pairs per handle) */
-    SFMB200_OPT_BATCH_PIPELINE = 11, /* whole-path calls on a batch: cut the pairs into this many chunks and generate the hypotheses
-                                      of later chunks on a side stream while earlier chunks are scored (same bits): 2..16 chunks;
-                                      -1 (default), 0, 1: off - measured on B200 the co-resident generation only time-shares the
-                                      FMA pipe with scoring (config 4: 42.41 vs 42.47 ms), see DESIGN.md */
     SFMB200_OPT_SAMPLER = 10,      /* sample rows drawn on the device (d_idx == NULL): 0 (default) 8 distinct indices per hypothesis,
                                       independent between hypotheses; 1 the reference's scheme (sfm.cu:95-104): ONE
                                       permutation of the point indices cut into disjoint groups of 8, which needs

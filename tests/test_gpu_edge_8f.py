@@ -86,7 +86,8 @@ def test_bundle_adjust_then_rest_of_the_api_still_consistent(pkg, O):
 def test_failed_run_does_not_corrupt_the_threshold_scale(pkg, O):
     """ADVICE r1: run_device / run_host used to commit the new threshold scale before the ingest was validated; a
     failing call then left corr_s / corr_dup at the old scale while pt_scale claimed the new one, and the next
-    estimate at that threshold scored mis-scaled points."""
+    estimate at that threshold scored mis-scaled points.  Every argument is validated before anything is enqueued,
+    so a failing call leaves the handle as it was."""
     import torch
 
     K, Kinv = O.reference_K()
@@ -99,12 +100,19 @@ def test_failed_run_does_not_corrupt_the_threshold_scale(pkg, O):
     fresh = pkg.BatchedPairs(K, Kinv, 1, n, H)
     fresh.run_device(d_px, H, 7, 4e-6)
     want4 = fresh.get_inlier_counts().cpu().numpy().copy()
+    launches = h.launch_count()
     big = torch.zeros((n + 100, 4), device="cuda")
     with pytest.raises(pkg.SfmError):
         h.run_device(big, H, 7, 4e-6)                       # n above max_points: must leave the handle untouched
     with pytest.raises(pkg.SfmError):
         h.lib.call("sfmb200_run_host", h._h, None, n, H, __import__("ctypes").c_uint64(7), __import__("ctypes").c_float(4e-6),
                    None, None, None, None, None)            # null input
+    with pytest.raises(pkg.SfmError):
+        h.run_device(d_px, H + 1, 7, 4e-6)                  # H above max_hypotheses, with a valid input
+    with pytest.raises(pkg.SfmError):
+        h.run_host(px, H + 1, 7, 4e-6)
+    assert h.launch_count() == launches                     # nothing was enqueued
+    assert np.array_equal(h.get_inlier_counts().cpu().numpy(), want)
     h.estimate_e(H, 7, 4e-6)                                # re-materialises the scaled copies for the new threshold
     assert np.array_equal(h.get_inlier_counts().cpu().numpy(), want4)
     h.estimate_e(H, 7, 1e-6)

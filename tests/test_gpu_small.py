@@ -104,37 +104,22 @@ def test_fused_path_host_entry_and_dispatch(pkg, O):
     h.close(); ref.close()
 
 
-def test_batched_pipeline_equals_serial(pkg, O):
-    """Whole-path calls on a batch cut the pairs into chunks and generate the hypotheses of later chunks on a side stream
-    while earlier chunks are scored (option 11).  Same kernels and per-pair seeds: every result must be bit-identical to
-    the serial order, for chunk counts that do and do not divide the batch."""
+def test_batched_pair_equals_single_pair_with_its_seed(pkg, O):
+    """Pairs of a batch are seeded by their absolute index: pair 33 of a batch, alone on a handle with that pair's seed,
+    reproduces its batched result."""
     import torch
 
     K, Kinv = O.reference_K()
     B, n, H = 70, 1200, 900
     px = np.stack([O.synthetic_pair(n, seed=300 + (b % 5))["px"] for b in range(B)])
-    d_px = torch.from_numpy(px).cuda()
     ref = pkg.BatchedPairs(K, Kinv, B, n, H)
     ref.set_option(OPT_SMALL, 0)
-    ref.set_option(11, 0)
-    ref.run_device(d_px, H, 42, THR)
-    want = (ref.get_best(), ref.get_E().copy(), ref.get_poses().copy(), ref.get_pose_index().copy(),
-            [ref.get_inlier_counts(b).cpu().numpy() for b in (0, 33, 69)], [ref.get_points_host(b) for b in (0, 33, 69)])
-    for chunks in (2, 7, 16):
-        h = pkg.BatchedPairs(K, Kinv, B, n, H)
-        h.set_option(OPT_SMALL, 0)
-        h.set_option(11, chunks)
-        for _ in range(2):                                   # twice: the side stream and its events are reused
-            h.run_device(d_px, H, 42, THR)
-        assert np.array_equal(h.get_best()[0], want[0][0]) and np.array_equal(h.get_best()[1], want[0][1])
-        assert np.array_equal(h.get_E(), want[1]) and np.array_equal(h.get_poses(), want[2]) and np.array_equal(h.get_pose_index(), want[3])
-        for k, b in enumerate((0, 33, 69)):
-            assert np.array_equal(h.get_inlier_counts(b).cpu().numpy(), want[4][k])
-            assert np.array_equal(h.get_points_host(b), want[5][k])
-        h.close()
-    # pairs of a batch are seeded by their absolute index: pair 33 alone with that seed reproduces its batched result
+    ref.run_device(torch.from_numpy(px).cuda(), H, 42, THR)
     one = pkg.BatchedPairs(K, Kinv, 1, n, H)
     one.set_option(OPT_SMALL, 0)
     one.run_device(torch.from_numpy(px[33]).cuda(), H, (42 + 0x632BE59BD9B4E019 * 33) % (1 << 64), THR)
-    assert np.array_equal(one.get_inlier_counts(0).cpu().numpy(), want[4][1])
+    assert np.array_equal(one.get_inlier_counts(0).cpu().numpy(), ref.get_inlier_counts(33).cpu().numpy())
+    with pytest.raises(pkg.SfmError) as e:
+        ref.set_option(11, 2)                              # the retired batch-pipeline option
+    assert e.value.code == -1
     one.close(); ref.close()

@@ -65,8 +65,6 @@ for n, H, pairs in ((2153, 269, 1), (900, 100, 3), (4100, 600, 1)):
     h.set_option(10, 1)
     h.estimate_e(min(H, n // 8), 5, 1e-6)
     h.set_option(10, 0)
-    h.set_option(11, 2)
-    h.run_device(torch.from_numpy(px).cuda(), H, 5, 1e-6)
     pkg.sharding.connect_peers(h, 0, 1)
     pkg.sharding.estimate_e_p2p(h, H, 5, 1e-6)
     pkg.sharding.estimate_e_p2p(h, H, 6, 1e-6)
