@@ -8,7 +8,7 @@ The product path is the C-ABI CUDA library ``libsfmb200.so`` (include/sfmb200.h)
 There is no CPU fallback: loading fails loudly when the library is missing.
 """
 from .binding import Lib, SfmError, load_library, lib_path  # noqa: F401
-from .image_pair import ImagePair, BatchedPairs  # noqa: F401
+from .image_pair import ImagePair, BatchedPairs, check_offsets, pack_ragged, unpack_ragged  # noqa: F401
 from . import sharding, synthetic  # noqa: F401
 
-__all__ = ["Lib", "SfmError", "load_library", "lib_path", "ImagePair", "BatchedPairs"]
+__all__ = ["Lib", "SfmError", "load_library", "lib_path", "ImagePair", "BatchedPairs", "check_offsets", "pack_ragged", "unpack_ragged"]

@@ -41,6 +41,10 @@ SIGNATURES = {
     "sfmb200_set_points_xy": (C.c_int, [_vp, _vp, C.c_int]),
     "sfmb200_set_points_xy_host": (C.c_int, [_vp, _vp, C.c_int]),
     "sfmb200_set_points_normalised": (C.c_int, [_vp, _vp, C.c_int]),
+    "sfmb200_set_points_xy_ragged": (C.c_int, [_vp, _vp, _vp]),
+    "sfmb200_run_device_ragged": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_uint64, C.c_float]),
+    "sfmb200_run_host_ragged": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_uint64, C.c_float, _vp, _vp, _vp, _vp, _vp]),
+    "sfmb200_get_point_counts": (C.c_int, [_vp, _vp]),
     "sfmb200_estimate_e": (C.c_int, [_vp, _vp, C.c_int, C.c_uint64, C.c_float]),
     "sfmb200_estimate_e_slice": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_float]),
     "sfmb200_copy_to_vbo_coloured": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_float, C.c_int, C.c_float, C.c_float]),

@@ -99,6 +99,14 @@ struct sfmb200_handle {
     float* host_header;    // pinned mirror of pack_header
     int* adapt;            // device [4]: adaptive termination flag, hypotheses used, pairs unsatisfied, spare
     void* arena;
+    // correspondence counts of the current points (set by every ingest) and the smallest per-pair count
+    PointCounts pc;
+    int n_min;
+    // per-pair-count mode: the counts table (RaggedTable), allocated by the first *_ragged ingest.  The pinned mirror is
+    // filled on the host and uploaded with one copy; ragged_ev marks that copy, the next fill waits for it.
+    void* ragged_host;
+    void* ragged_dev;
+    cudaEvent_t ragged_ev;
     // optional per-stage timing (SFMB200_OPT_PROFILE): ring of event sets, one set
     // per run_device / run_host call, 8 boundary marks -> 7 stage durations
     int profile;
@@ -108,6 +116,34 @@ struct sfmb200_handle {
     unsigned char* prof_mask;     // [PROF_RING] bit k = mark k recorded
 };
 static const int PROF_RING = 256;
+
+// Counts table of a batch with per-pair counts, one block in the same layout on the host and on the device:
+// grain_off [B + 1] (DeviceState::grain_off), n_pair [B] (DeviceState::n_pair), row_off [B + 1] (first packed row per pair).
+struct RaggedTable {
+    long long* grain_off;
+    int* n_pair;
+    int* row_off;
+    static size_t bytes(int B) { return (size_t)(B + 1) * sizeof(long long) + (size_t)B * sizeof(int) + (size_t)(B + 1) * sizeof(int); }
+    static RaggedTable at(void* base, int B) {
+        RaggedTable r;
+        r.grain_off = (long long*)base;
+        r.n_pair = (int*)(r.grain_off + B + 1);
+        r.row_off = r.n_pair + B;
+        return r;
+    }
+};
+static bool is_ragged(const sfmb200_handle* h) { return h->s.n_pair != nullptr; }
+// Correspondences of pair b on the host side (getters, packed outputs).
+static int host_pair_n(const sfmb200_handle* h, int b) {
+    return is_ragged(h) ? RaggedTable::at(h->ragged_host, h->s.B).n_pair[b] : h->s.n;
+}
+// Stages that need the same number of correspondences in every pair refuse a handle in per-pair-count mode.
+static int refuse_ragged(const sfmb200_handle* h, const char* stage) {
+    if (!is_ragged(h)) return SFMB200_OK;
+    char msg[256];
+    snprintf(msg, sizeof(msg), "%s needs the same number of correspondences in every pair; the last ingest was *_ragged", stage);
+    return fail(SFMB200_ERR_STATE, msg);
+}
 static inline void prof_mark(sfmb200_handle* h, int k) {
     if (!h->profile) return;
     cudaEventRecord(h->prof_ev[h->prof_cur][k], h->stream);
@@ -203,13 +239,15 @@ static int lazy_arena(sfmb200_handle* h, void** arena, Layout layout) {
 static void release(sfmb200_handle* h) {
     if (h->own_stream) cudaStreamDestroy(h->stream);
     if (h->host_header) cudaFreeHost(h->host_header);
+    if (h->ragged_host) cudaFreeHost(h->ragged_host);
+    if (h->ragged_ev) cudaEventDestroy(h->ragged_ev);
     if (h->prof_ev) {
         for (int i = 0; i < PROF_RING; i++)
             for (int k = 0; k < 8; k++) cudaEventDestroy(h->prof_ev[i][k]);
         delete[] h->prof_ev;
         delete[] h->prof_mask;
     }
-    for (void* p : {h->arena, h->chain_arena, h->gba_arena, h->ba_arena, (void*)h->px_staging, (void*)h->pack_points})
+    for (void* p : {h->arena, h->chain_arena, h->gba_arena, h->ba_arena, (void*)h->px_staging, (void*)h->pack_points, h->ragged_dev})
         if (p) cudaFree(p);
     delete h;
 }
@@ -380,13 +418,22 @@ static int check_n(sfmb200_t* h, const void* p, int n) {
     if (n < 8 || n > h->s.n_max) return fail(SFMB200_ERR_ARG, "n must be in [8, max_points]");
     return SFMB200_OK;
 }
+// Every uniform ingest commits its n through here, which also returns the handle to uniform mode.
+static void set_uniform(sfmb200_handle* h, int n) {
+    h->s.n = n;
+    h->s.n_pair = nullptr;
+    h->s.grain_off = nullptr;
+    const long long B = h->s.B;
+    h->pc = PointCounts{h->s.B, n, B * n, B * ((n + SCORE_GRAIN - 1) / SCORE_GRAIN), false};
+    h->n_min = n;
+}
 
 int sfmb200_set_points_sift(sfmb200_t* h, const void* d_sift, int n) {
     ENTER(h);
     int rc = check_n(h, d_sift, n);
     if (rc) return rc;
     if (h->s.B != 1) return fail(SFMB200_ERR_ARG, "SiftPoint ingest needs pairs == 1");
-    h->s.n = n;
+    set_uniform(h, n);
     launch_ingest_sift(h->s, d_sift, n, h->stream);
     CKL();
     h->launches++;
@@ -410,7 +457,7 @@ int sfmb200_set_points_sift_filtered(sfmb200_t* h, const void* d_sift, int n, fl
     CK(cudaStreamSynchronize(h->stream));
     if (h_kept) *h_kept = kept;
     if (kept < 8) return fail(SFMB200_ERR_STATE, "fewer than 8 correspondences survive the match filter");
-    h->s.n = kept;
+    set_uniform(h, kept);
     h->st.new_points();
     return SFMB200_OK;
 }
@@ -420,7 +467,7 @@ int sfmb200_set_points_sift_filtered(sfmb200_t* h, const void* d_sift, int n, fl
 static int ingest_xy(sfmb200_t* h, const float* d_px, int n, float scale) {
     int rc = check_n(h, d_px, n);
     if (rc) return rc;
-    h->s.n = n;
+    set_uniform(h, n);
     if (scale > 0.0f) h->s.pt_scale = scale;
     prof_mark(h, 0);
     launch_ingest_xy(h->s, d_px, n, h->stream);
@@ -436,26 +483,90 @@ int sfmb200_set_points_xy(sfmb200_t* h, const float* d_px, int n) {
 }
 // Device copy of host input that the kernels cannot reach directly (pageable, or larger than the zero-copy limit): the
 // staging buffer is allocated on first use, so device-resident workflows (run_device, the batched configs) never pay for it.
-static int stage_input(sfmb200_handle* h, const float* h_px, int n) {
+// rows: correspondences in h_px, packed (at most pairs * max_points).
+static int stage_input(sfmb200_handle* h, const float* h_px, long long rows) {
     if (!h->px_staging) CK(cudaMalloc(&h->px_staging, (size_t)h->s.B * h->s.n_stride * 4 * sizeof(float)));
-    CK(cudaMemcpyAsync(h->px_staging, h_px, (size_t)h->s.B * n * 4 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->px_staging, h_px, (size_t)rows * 4 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     return SFMB200_OK;
 }
 int sfmb200_set_points_xy_host(sfmb200_t* h, const float* h_px, int n) {
     ENTER(h);
     if (int rc = check_n(h, h_px, n)) return rc;
-    if (int rc = stage_input(h, h_px, n)) return rc;
+    if (int rc = stage_input(h, h_px, (long long)h->s.B * n)) return rc;
     return ingest_xy(h, h->px_staging, n, 0.0f);
 }
 int sfmb200_set_points_normalised(sfmb200_t* h, const float* d_x, int n) {
     ENTER(h);
     int rc = check_n(h, d_x, n);
     if (rc) return rc;
-    h->s.n = n;
+    set_uniform(h, n);
     launch_ingest_normalised(h->s, d_x, n, h->stream);
     CKL();
     h->launches++;
     h->st.new_points();
+    return SFMB200_OK;
+}
+
+// ---- per-pair counts: packed rows, pair b owns rows [offs[b], offs[b + 1]) ----
+static int check_ragged(sfmb200_t* h, const void* px, const int32_t* offs) {
+    if (!h || !px || !offs) return fail(SFMB200_ERR_ARG, "null argument");
+    if (offs[0] != 0) return fail(SFMB200_ERR_ARG, "offsets[0] must be 0");
+    for (int b = 0; b < h->s.B; b++) {
+        const long long c = (long long)offs[b + 1] - offs[b];
+        if (c < 0) return fail(SFMB200_ERR_ARG, "offsets must not decrease");
+        if (c < 8 || c > h->s.n_max) return fail(SFMB200_ERR_ARG, "every count offsets[b+1] - offsets[b] must be in [8, max_points]");
+    }
+    return SFMB200_OK;
+}
+// Validated offsets: fills the counts table, uploads it and launches the ingest.  `scale` as for ingest_xy.
+static int ingest_ragged(sfmb200_t* h, const float* d_px, const int32_t* offs, float scale) {
+    DeviceState& s = h->s;
+    const int B = s.B;
+    const size_t bytes = RaggedTable::bytes(B);
+    if (!h->ragged_dev) CK(cudaMalloc(&h->ragged_dev, bytes));
+    if (!h->ragged_host) CK(cudaMallocHost(&h->ragged_host, bytes));
+    if (!h->ragged_ev) CK(cudaEventCreateWithFlags(&h->ragged_ev, cudaEventDisableTiming));
+    CK(cudaEventSynchronize(h->ragged_ev));      // the previous upload has read the mirror
+    const RaggedTable m = RaggedTable::at(h->ragged_host, B), d = RaggedTable::at(h->ragged_dev, B);
+    long long grains = 0, sum = 0;
+    int n_max = 0, n_min = s.n_max;
+    m.grain_off[0] = 0;
+    for (int b = 0; b < B; b++) {
+        const int c = offs[b + 1] - offs[b];
+        m.n_pair[b] = c;
+        m.row_off[b] = offs[b];
+        grains += (c + SCORE_GRAIN - 1) / SCORE_GRAIN;
+        m.grain_off[b + 1] = grains;
+        sum += c;
+        n_max = c > n_max ? c : n_max;
+        n_min = c < n_min ? c : n_min;
+    }
+    m.row_off[B] = offs[B];
+    CK(cudaMemcpyAsync(h->ragged_dev, h->ragged_host, bytes, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaEventRecord(h->ragged_ev, h->stream));
+    s.n = n_max;
+    s.n_pair = d.n_pair;
+    s.grain_off = d.grain_off;
+    h->pc = PointCounts{B, n_max, sum, grains, true};
+    h->n_min = n_min;
+    if (scale > 0.0f) s.pt_scale = scale;
+    prof_mark(h, 0);
+    launch_ingest_xy_ragged(s, d_px, d.row_off, h->stream);
+    prof_mark(h, 1);
+    CKL();
+    h->launches++;
+    h->st.new_points();
+    return SFMB200_OK;
+}
+int sfmb200_set_points_xy_ragged(sfmb200_t* h, const float* d_px, const int32_t* h_offsets) {
+    ENTER(h);
+    if (int rc = check_ragged(h, d_px, h_offsets)) return rc;
+    return ingest_ragged(h, d_px, h_offsets, 0.0f);
+}
+int sfmb200_get_point_counts(sfmb200_t* h, int32_t* h_counts) {
+    ENTER(h);
+    if (!h || !h_counts) return fail(SFMB200_ERR_ARG, "null argument");
+    for (int b = 0; b < h->s.B; b++) h_counts[b] = host_pair_n(h, b);
     return SFMB200_OK;
 }
 
@@ -474,19 +585,21 @@ static int ensure_scaled(sfmb200_handle* h, float scale) {
 // Scoring launch of the essential-matrix model with the handle's metric: Sampson error (the tuned kernel family) or
 // symmetric epipolar distance (same kernel, MODEL = 2, in the three tile sizes).  h->plan must be set.
 static void score_essential(sfmb200_handle* h, const DeviceState& s, int H, int h_offset, float thr) {
-    if (s.metric == 0) launch_score(s, h->plan, H, h_offset, thr, h->stream);
-    else launch_score_symmetric(s, h->plan, H, h_offset, thr, h->stream);
+    const int* h_n_pair = is_ragged(h) ? RaggedTable::at(h->ragged_host, s.B).n_pair : nullptr;
+    if (s.metric == 0) launch_score(s, h->plan, H, h_offset, thr, h_n_pair, h->stream);
+    else launch_score_symmetric(s, h->plan, H, h_offset, thr, h_n_pair, h->stream);
 }
-static ScorePlan plan_essential(const sfmb200_handle* h, int n, int H) {
-    return h->s.metric == 0 ? make_score_plan(h->s.B, n, H, h->score_variant, h->sms) : make_score_plan_homography(h->s.B, n, H, h->sms);
+static ScorePlan plan_essential(const sfmb200_handle* h, int H) {
+    return h->s.metric == 0 ? make_score_plan(h->pc, H, h->score_variant, h->sms) : make_score_plan_homography(h->pc, H, h->sms);
 }
 
 // The fused single-launch path (small.cu) serves essential-matrix estimates with the projector solver whose
 // hypotheses fit one cluster's shared memory; `pose`: the call also runs the pose stage, which the fused kernel
 // implements in reference (compat) semantics only.  Not used while per-stage events are being recorded.
 constexpr int SMALL_PATH_MAX_PAIRS = 4;
-static bool small_path_ok(const sfmb200_handle* h, int n, int H, bool pose) {
-    if (h->small_path == 0 || h->profile || h->hyp_solver != 1 || h->s.skip != nullptr || h->s.metric != 0) return false;
+// `ragged`: the points are (or are about to be) held with per-pair counts, which the fused kernel does not take.
+static bool small_path_ok(const sfmb200_handle* h, int n, int H, bool pose, bool ragged) {
+    if (ragged || h->small_path == 0 || h->profile || h->hyp_solver != 1 || h->s.skip != nullptr || h->s.metric != 0) return false;
     if (h->score_variant >= 0 && h->small_path != 1) return false;      // the caller asked for a specific scoring kernel
     if (pose && !h->compat) return false;
     if (H > small_path_max_hypotheses()) return false;
@@ -504,20 +617,20 @@ int sfmb200_estimate_e_slice(sfmb200_t* h, const int32_t* d_idx, int H_total, in
     if (H < 1 || H > h->s.h_max || h_begin < 0 || (long long)h_begin + H > (long long)H_total)
         return fail(SFMB200_ERR_ARG, "hypothesis slice out of range / above max_hypotheses");
     if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive");
-    if (!d_idx && h->s.sampler == 1 && 8ll * H_total > (long long)h->s.n)
-        return fail(SFMB200_ERR_ARG, "the disjoint-permutation sampler needs 8 * H_total <= n (the reference uses H = N / 8)");
+    if (!d_idx && h->s.sampler == 1 && 8ll * H_total > (long long)h->n_min)
+        return fail(SFMB200_ERR_ARG, "the disjoint-permutation sampler needs 8 * H_total <= n, in every pair (the reference uses H = N / 8)");
     h->H = H;
     h->h_begin = h_begin;
     h->thr = thr;
     if (int rc = ensure_scaled(h, make_thr_scale(thr).ik)) return rc;
-    if (small_path_ok(h, h->s.n, H, false)) {
+    if (small_path_ok(h, h->s.n, H, false, is_ragged(h))) {
         // hypothesis generation + scoring + arg-max + selection in one cluster launch
         CK(launch_small_path(h->s, nullptr, d_idx, (long long)H_total * 8, H, h_begin, seed, thr, h->compat, 0, SMALL_ESTIMATE, h->stream));
         memset(&h->plan, 0, sizeof(h->plan));
         h->plan.variant = -2;      // reported by sfmb200_score_plan: the fused path
         h->launches += 1;
     } else {
-        h->plan = plan_essential(h, h->s.n, H);
+        h->plan = plan_essential(h, H);
         launch_hypgen(h->s, d_idx, (long long)H_total * 8, H, h_begin, seed, h->hyp_solver, h->stream);
         prof_mark(h, 2);
         CKL();
@@ -535,6 +648,7 @@ int sfmb200_estimate_e_slice(sfmb200_t* h, const int32_t* d_idx, int H_total, in
 
 int sfmb200_find_homography(sfmb200_t* h, int loops, uint64_t seed, float thresh, float* h_H, int32_t* h_matches) {
     ENTER_HANDLE(h);
+    if (int rc = refuse_ragged(h, "find_homography")) return rc;
     if (int rc = need(h, NEED_POINTS, "find_homography before set_points")) return rc;
     if (loops < 1 || loops > h->s.h_max) return fail(SFMB200_ERR_ARG, "loops out of range / above max_hypotheses");
     if (!(thresh > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive");
@@ -554,7 +668,7 @@ int sfmb200_find_homography(sfmb200_t* h, int loops, uint64_t seed, float thresh
     h->H = loops;
     h->h_begin = 0;
     h->thr = thr2;
-    h->plan = make_score_plan_homography(h->s.B, h->s.n, loops, h->sms);
+    h->plan = make_score_plan_homography(h->pc, loops, h->sms);
     launch_hypgen(h->s, nullptr, (long long)loops * 8, loops, 0, seed, 2, h->stream);
     CKL();
     launch_score_homography(h->s, h->plan, loops, 0, thr2, h->stream);
@@ -627,7 +741,7 @@ int sfmb200_estimate_e_adaptive(sfmb200_t* h, const int32_t* d_idx, int H_max, i
     while (lo < H_max) {
         if (hi > H_max) hi = H_max;
         const int Hr = (int)(hi - lo);
-        h->plan = plan_essential(h, s.n, Hr);
+        h->plan = plan_essential(h, Hr);
         launch_hypgen(s, d_idx, (long long)H_max * 8, Hr, (int)lo, seed, h->hyp_solver, h->stream, rounds > 0);
         CKL();
         score_essential(h, s, Hr, (int)lo, thr);
@@ -754,6 +868,7 @@ int sfmb200_mg_close(sfmb200_t* h) {
 // H_total hypotheses, exchanges the packed winners through peer memory and takes the global winner's E.
 int sfmb200_estimate_e_mg(sfmb200_t* h, const int32_t* d_idx, int H_total, uint64_t seed, float thr) {
     ENTER_HANDLE(h);
+    if (int rc = refuse_ragged(h, "estimate_e_mg")) return rc;
     if (!h->mg_connected) return fail(SFMB200_ERR_STATE, "estimate_e_mg before mg_init / mg_connect");
     if (*(volatile int*)h->mg_failed_host != 0) {
         h->st.lose_essential();
@@ -796,6 +911,7 @@ int sfmb200_best_buffer(sfmb200_t* h, uint64_t** d_best) {
 }
 int sfmb200_adopt_best(sfmb200_t* h, const int32_t* d_idx, int H_total, uint64_t seed) {
     ENTER_HANDLE(h);
+    if (int rc = refuse_ragged(h, "adopt_best")) return rc;
     if (int rc = need(h, NEED_POINTS, "adopt_best before set_points")) return rc;
     if (h->st.E == Held::homography || !(h->thr > 0.0f))
         return fail(SFMB200_ERR_STATE, "adopt_best follows an essential-matrix estimate (estimate_e / estimate_e_slice) on this handle");
@@ -808,6 +924,7 @@ int sfmb200_adopt_best(sfmb200_t* h, const int32_t* d_idx, int H_total, uint64_t
 
 int sfmb200_refine_e(sfmb200_t* h, int iterations) {
     ENTER_HANDLE(h);
+    if (int rc = refuse_ragged(h, "refine_e")) return rc;
     if (iterations < 0 || iterations > 64) return fail(SFMB200_ERR_ARG, "iterations must be in [0, 64]");
     if (int rc = need(h, NEED_POINTS | NEED_ESSENTIAL, "refine_e before an essential matrix exists")) return rc;
     if (iterations == 0) return SFMB200_OK;
@@ -845,6 +962,7 @@ static int ensure_ba_arena(sfmb200_handle* h) {
 // inliers of the refined E, spare - of the LAST round.
 int sfmb200_bundle_adjust(sfmb200_t* h, int outer_rounds, int iterations, float* h_stats) {
     ENTER_HANDLE(h);
+    if (int rc = refuse_ragged(h, "bundle_adjust")) return rc;
     if (outer_rounds < 1 || outer_rounds > 64 || iterations < 1 || iterations > 256)
         return fail(SFMB200_ERR_ARG, "outer_rounds in [1, 64] and iterations in [1, 256] required");
     if (int rc = need(h, NEED_POINTS | NEED_ESSENTIAL | NEED_POSE, "bundle_adjust needs an essential matrix and a chosen pose"))
@@ -864,6 +982,7 @@ int sfmb200_bundle_adjust(sfmb200_t* h, int outer_rounds, int iterations, float*
 // N-view chaining (chain.cu): pairs of the handle = consecutive view pairs over index-aligned tracks.
 int sfmb200_chain_views(sfmb200_t* h, float* d_cloud, int32_t* d_count, float* h_cameras, float* h_scales, int32_t* h_used) {
     ENTER_HANDLE(h);
+    if (int rc = refuse_ragged(h, "chain_views")) return rc;
     if (h->s.B > 256) return fail(SFMB200_ERR_ARG, "chain_views handles at most 256 pairs (257 views)");
     if (int rc = need(h, NEED_POINTS | NEED_ESSENTIAL | NEED_POSE,
                       "chain_views needs an essential matrix, a chosen pose and triangulated points per pair"))
@@ -896,6 +1015,7 @@ int sfmb200_bundle_adjust_global(sfmb200_t* h, float* d_cloud, const int32_t* d_
                                  float* h_stats) {
     ENTER(h);
     if (!h || !d_cloud || !d_count) return fail(SFMB200_ERR_ARG, "null argument");
+    if (int rc = refuse_ragged(h, "bundle_adjust_global")) return rc;
     if (iterations < 1 || iterations > 1000) return fail(SFMB200_ERR_ARG, "iterations must be in [1, 1000]");
     if (h->s.B > GBA_MAX_PAIRS) return fail(SFMB200_ERR_ARG, "bundle_adjust_global handles at most 16 pairs (17 views)");
     if (int rc = need(h, NEED_CHAIN | NEED_POINTS | NEED_ESSENTIAL | NEED_POSE,
@@ -970,7 +1090,7 @@ static int run_stages(sfmb200_t* h, int H, uint64_t seed, float thr) {
     h->h_begin = 0;
     h->thr = thr;
     if (int rc = ensure_scaled(h, make_thr_scale(thr).ik)) return rc;     // no-op after run_device / run_host's own ingest
-    h->plan = plan_essential(h, h->s.n, H);
+    h->plan = plan_essential(h, H);
     launch_hypgen(h->s, nullptr, (long long)H * 8, H, 0, seed, h->hyp_solver, h->stream);
     prof_mark(h, 2);
     CKL();
@@ -996,7 +1116,7 @@ static int run_stages(sfmb200_t* h, int H, uint64_t seed, float thr) {
 // Whole path in ONE launch (small.cu), for the problems small_path_ok admits.  d_px: device-readable pixel
 // correspondences.
 static int run_small(sfmb200_t* h, const float* d_px, int n, int H, uint64_t seed, float thr) {
-    h->s.n = n;
+    set_uniform(h, n);
     h->s.pt_scale = make_thr_scale(thr).ik;
     cudaError_t e = launch_small_path(h->s, d_px, nullptr, (long long)H * 8, H, 0, seed, thr, h->compat, h->tri_inliers_only,
                                       SMALL_INGEST | SMALL_ESTIMATE | SMALL_POSE | SMALL_TRI, h->stream);
@@ -1013,11 +1133,11 @@ static int run_small(sfmb200_t* h, const float* d_px, int n, int H, uint64_t see
     return SFMB200_OK;
 }
 
-// Arguments of run_device / run_host.  All are checked before anything is enqueued, so a call that fails here leaves
-// the handle as it was.
-static int check_run(sfmb200_t* h, const void* px, int n, int H, float thr) {
+// Arguments of run_device / run_host and their *_ragged forms (offs != nullptr: n is not used).  All are checked before
+// anything is enqueued, so a call that fails here leaves the handle as it was.
+static int check_run(sfmb200_t* h, const void* px, int n, const int32_t* offs, int H, float thr) {
     if (!(thr > 0.0f)) return fail(SFMB200_ERR_ARG, "threshold must be positive");
-    if (int rc = check_n(h, px, n)) return rc;
+    if (int rc = offs ? check_ragged(h, px, offs) : check_n(h, px, n)) return rc;
     if (H < 1 || H > h->s.h_max) return fail(SFMB200_ERR_ARG, "H out of range / above max_hypotheses");
     return SFMB200_OK;
 }
@@ -1025,22 +1145,33 @@ static int check_run(sfmb200_t* h, const void* px, int n, int H, float thr) {
 // The whole path on validated arguments and device-readable pixel correspondences: the fused single launch when the
 // problem is small, else the ingest followed by the five-launch path.
 static int run_path(sfmb200_t* h, const float* d_px, int n, int H, uint64_t seed, float thr) {
-    if (small_path_ok(h, n, H, true)) return run_small(h, d_px, n, H, seed, thr);
+    if (small_path_ok(h, n, H, true, false)) return run_small(h, d_px, n, H, seed, thr);
     if (int rc = ingest_xy(h, d_px, n, make_thr_scale(thr).ik)) return rc;     // writes the scaled copies for this threshold
+    return run_stages(h, H, seed, thr);
+}
+static int run_path_ragged(sfmb200_t* h, const float* d_px, const int32_t* offs, int H, uint64_t seed, float thr) {
+    if (int rc = ingest_ragged(h, d_px, offs, make_thr_scale(thr).ik)) return rc;
     return run_stages(h, H, seed, thr);
 }
 
 int sfmb200_run_device(sfmb200_t* h, const float* d_px, int n, int H, uint64_t seed, float thr) {
     ENTER_HANDLE(h);
-    if (int rc = check_run(h, d_px, n, H, thr)) return rc;
+    if (int rc = check_run(h, d_px, n, nullptr, H, thr)) return rc;
     prof_next(h);
     return run_path(h, d_px, n, H, seed, thr);
+}
+int sfmb200_run_device_ragged(sfmb200_t* h, const float* d_px, const int32_t* h_offsets, int H, uint64_t seed, float thr) {
+    ENTER_HANDLE(h);
+    if (int rc = check_run(h, d_px, 0, h_offsets, H, thr)) return rc;
+    prof_next(h);
+    return run_path_ragged(h, d_px, h_offsets, H, seed, thr);
 }
 
 // Results of the whole path packed for the host: one small header per pair and a
 // compact [4][n] copy of the points, so run_host needs two DMA transfers instead
 // of six (each small D2H copy costs ~5-10 us of latency on the critical path).
-__global__ void pack_results_kernel(DeviceState s, float* header, float* points, int want_points) {
+// row_off (per-pair counts): pair b's [4][n_b] block starts at float 4 * row_off[b]; nullptr: at b * 4 * n.
+__global__ void pack_results_kernel(DeviceState s, float* header, float* points, const int* row_off, int want_points) {
     const int b = blockIdx.y;
     if (blockIdx.x == 0 && threadIdx.x < 32) {
         const int t = threadIdx.x;
@@ -1054,11 +1185,12 @@ __global__ void pack_results_kernel(DeviceState s, float* header, float* points,
     }
     if (!want_points) return;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= s.n) return;
+    const int n = pair_n(s, b);
+    if (i >= n) return;
     const float* in = s.points + (size_t)b * 4 * s.n_stride;
-    float* out = points + (size_t)b * 4 * s.n;
+    float* out = points + (row_off ? 4 * (size_t)row_off[b] : (size_t)b * 4 * n);
 #pragma unroll
-    for (int r = 0; r < 4; r++) out[(size_t)r * s.n + i] = in[(size_t)r * s.n_stride + i];
+    for (int r = 0; r < 4; r++) out[(size_t)r * n + i] = in[(size_t)r * s.n_stride + i];
 }
 
 // Device-visible alias of a host pointer when it is page-locked (cudaHostAlloc / cudaHostRegister / torch
@@ -1074,33 +1206,35 @@ static void* pinned_alias(const void* host) {
     return a.type == cudaMemoryTypeHost ? a.devicePointer : nullptr;
 }
 
-int sfmb200_run_host(sfmb200_t* h, const float* h_px, int n, int H, uint64_t seed, float thr, float* h_E, float* h_P,
-                     int32_t* h_pose_index, int32_t* h_inliers, float* h_points) {
-    ENTER_HANDLE(h);
-    if (int rc = check_run(h, h_px, n, H, thr)) return rc;
-    prof_next(h);
-    // zero copy pays where latency dominates (config-2-sized calls: 160 KB each way); bulk transfers (batched
-    // config 4: hundreds of MB) stay with the copy engines, which keep more PCIe requests in flight than a kernel
-    const size_t zero_copy_limit = 4u << 20;
-    const size_t in_bytes = (size_t)h->s.B * n * 4 * sizeof(float);
-    const float* d_px = in_bytes <= zero_copy_limit ? (const float*)pinned_alias(h_px) : nullptr;
-    if (!d_px) {          // pageable, or too large for zero copy: one copy into the staging buffer
-        if (int rc = stage_input(h, h_px, n)) return rc;
-        d_px = h->px_staging;
+// zero copy pays where latency dominates (config-2-sized calls: 160 KB each way); bulk transfers (batched
+// config 4: hundreds of MB) stay with the copy engines, which keep more PCIe requests in flight than a kernel
+constexpr size_t ZERO_COPY_LIMIT = 4u << 20;
+
+// Device-readable form of run_host*'s input of `rows` packed correspondences: a pinned alias, or the staging copy.
+static int host_input(sfmb200_handle* h, const float* h_px, long long rows, const float** d_px) {
+    *d_px = (size_t)rows * 4 * sizeof(float) <= ZERO_COPY_LIMIT ? (const float*)pinned_alias(h_px) : nullptr;
+    if (!*d_px) {          // pageable, or too large for zero copy: one copy into the staging buffer
+        if (int rc = stage_input(h, h_px, rows)) return rc;
+        *d_px = h->px_staging;
     }
-    if (int rc = run_path(h, d_px, n, H, seed, thr)) return rc;
+    return SFMB200_OK;
+}
+
+// Results of run_host* to the host after the path ran: `rows` points in all; row_off as for pack_results_kernel.
+static int host_results(sfmb200_handle* h, long long rows, const int* row_off, float* h_E, float* h_P, int32_t* h_pose_index,
+                        int32_t* h_inliers, float* h_points) {
     DeviceState& s = h->s;
-    const size_t B = s.B;
-    float* pts_alias = B * 4 * (size_t)s.n * sizeof(float) <= zero_copy_limit ? (float*)pinned_alias(h_points) : nullptr;
+    const size_t B = s.B, pts_bytes = (size_t)rows * 4 * sizeof(float);
+    float* pts_alias = pts_bytes <= ZERO_COPY_LIMIT ? (float*)pinned_alias(h_points) : nullptr;
     if (h_points && !pts_alias && !h->pack_points) CK(cudaMalloc(&h->pack_points, B * 4 * (size_t)s.n_max * sizeof(float)));
     dim3 grid(h_points ? (s.n + 255) / 256 : 1, (unsigned)B);
     // header: always through the handle's own pinned buffer (device-visible under UVA); points: straight into the
     // caller's buffer when it is pinned, else into the device staging copy followed by one DMA
-    pack_results_kernel<<<grid, 256, 0, h->stream>>>(s, h->host_header, pts_alias ? pts_alias : h->pack_points, h_points ? 1 : 0);
+    pack_results_kernel<<<grid, 256, 0, h->stream>>>(s, h->host_header, pts_alias ? pts_alias : h->pack_points, row_off,
+                                                     h_points ? 1 : 0);
     CKL();
     h->launches++;
-    if (h_points && !pts_alias)
-        CK(cudaMemcpyAsync(h_points, h->pack_points, B * 4 * (size_t)s.n * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    if (h_points && !pts_alias) CK(cudaMemcpyAsync(h_points, h->pack_points, pts_bytes, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     for (size_t b = 0; b < B; b++) {
         const float* hd = h->host_header + b * 32;
@@ -1110,6 +1244,29 @@ int sfmb200_run_host(sfmb200_t* h, const float* h_px, int n, int H, uint64_t see
         if (h_inliers) memcpy(h_inliers + b, hd + 26, sizeof(int32_t));
     }
     return SFMB200_OK;
+}
+
+int sfmb200_run_host(sfmb200_t* h, const float* h_px, int n, int H, uint64_t seed, float thr, float* h_E, float* h_P,
+                     int32_t* h_pose_index, int32_t* h_inliers, float* h_points) {
+    ENTER_HANDLE(h);
+    if (int rc = check_run(h, h_px, n, nullptr, H, thr)) return rc;
+    prof_next(h);
+    const long long rows = (long long)h->s.B * n;
+    const float* d_px = nullptr;
+    if (int rc = host_input(h, h_px, rows, &d_px)) return rc;
+    if (int rc = run_path(h, d_px, n, H, seed, thr)) return rc;
+    return host_results(h, rows, nullptr, h_E, h_P, h_pose_index, h_inliers, h_points);
+}
+int sfmb200_run_host_ragged(sfmb200_t* h, const float* h_px, const int32_t* h_offsets, int H, uint64_t seed, float thr,
+                            float* h_E, float* h_P, int32_t* h_pose_index, int32_t* h_inliers, float* h_points) {
+    ENTER_HANDLE(h);
+    if (int rc = check_run(h, h_px, 0, h_offsets, H, thr)) return rc;
+    prof_next(h);
+    const long long rows = h_offsets[h->s.B];
+    const float* d_px = nullptr;
+    if (int rc = host_input(h, h_px, rows, &d_px)) return rc;
+    if (int rc = run_path_ragged(h, d_px, h_offsets, H, seed, thr)) return rc;
+    return host_results(h, rows, RaggedTable::at(h->ragged_dev, h->s.B).row_off, h_E, h_P, h_pose_index, h_inliers, h_points);
 }
 
 int sfmb200_copy_to_vbo(sfmb200_t* h, int pair, float* d_pos, float* d_col) {
@@ -1184,8 +1341,9 @@ int sfmb200_get_points(sfmb200_t* h, int pair, float* d_points) {
     int rc = check_pair(h, pair, d_points);
     if (rc) return rc;
     const DeviceState& s = h->s;
-    CK(cudaMemcpy2DAsync(d_points, (size_t)s.n * sizeof(float), s.points + (size_t)pair * 4 * s.n_stride,
-                         (size_t)s.n_stride * sizeof(float), (size_t)s.n * sizeof(float), 4, cudaMemcpyDeviceToDevice,
+    const size_t n = host_pair_n(h, pair);
+    CK(cudaMemcpy2DAsync(d_points, n * sizeof(float), s.points + (size_t)pair * 4 * s.n_stride,
+                         (size_t)s.n_stride * sizeof(float), n * sizeof(float), 4, cudaMemcpyDeviceToDevice,
                          h->stream));
     return SFMB200_OK;
 }
@@ -1194,8 +1352,9 @@ int sfmb200_get_points_host(sfmb200_t* h, int pair, float* h_points) {
     int rc = check_pair(h, pair, h_points);
     if (rc) return rc;
     const DeviceState& s = h->s;
-    CK(cudaMemcpy2DAsync(h_points, (size_t)s.n * sizeof(float), s.points + (size_t)pair * 4 * s.n_stride,
-                         (size_t)s.n_stride * sizeof(float), (size_t)s.n * sizeof(float), 4, cudaMemcpyDeviceToHost,
+    const size_t n = host_pair_n(h, pair);
+    CK(cudaMemcpy2DAsync(h_points, n * sizeof(float), s.points + (size_t)pair * 4 * s.n_stride,
+                         (size_t)s.n_stride * sizeof(float), n * sizeof(float), 4, cudaMemcpyDeviceToHost,
                          h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return SFMB200_OK;

@@ -24,6 +24,15 @@ __global__ void ingest_xy_kernel(DeviceState s, const float4* __restrict__ px, i
     float4 p = __ldg(px + (size_t)b * n + i);
     normalise_store(s, b, i, p.x, p.y, p.z, p.w, k);
 }
+// Packed rows: pair b's s.n_pair[b] rows start at row row_off[b].
+__global__ void ingest_xy_ragged_kernel(DeviceState s, const float4* __restrict__ px, const int* __restrict__ row_off, Mat9 k) {
+    pdl_trigger();
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    int b = blockIdx.y;
+    if (i >= s.n_pair[b]) return;
+    float4 p = __ldg(px + (size_t)row_off[b] + i);
+    normalise_store(s, b, i, p.x, p.y, p.z, p.w, k);
+}
 // ---------------------------------------------------------------------------
 // Ingest with match filtering (SURVEY.md 8f rank 1).  The reference feeds every
 // SIFT point of image 1 to the estimator unfiltered (main.cpp:298-299; its
@@ -102,7 +111,7 @@ sift_filter_scatter_kernel(DeviceState s, const float* __restrict__ sift, int n,
 // Re-materialise the scaled copies after the threshold (or the model) changed without a new ingest.
 __global__ void rescale_points_kernel(DeviceState s) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= s.n) return;
+    if (i >= pair_n(s, blockIdx.y)) return;
     size_t o = (size_t)blockIdx.y * s.n_stride + i;
     float4 p = s.corr[o];
     store_scaled(s, o, p.x, p.y, p.z, p.w);
@@ -132,6 +141,12 @@ void launch_ingest_xy(const DeviceState& s, const float* d_px, int n, cudaStream
     for (int i = 0; i < 9; i++) k.v[i] = s.Kinv[i];
     dim3 grid((n + 255) / 256, s.B);
     ingest_xy_kernel<<<grid, 256, 0, st>>>(s, (const float4*)d_px, n, k);
+}
+void launch_ingest_xy_ragged(const DeviceState& s, const float* d_px, const int* d_row_off, cudaStream_t st) {
+    Mat9 k;
+    for (int i = 0; i < 9; i++) k.v[i] = s.Kinv[i];
+    dim3 grid((s.n + 255) / 256, s.B);
+    ingest_xy_ragged_kernel<<<grid, 256, 0, st>>>(s, (const float4*)d_px, d_row_off, k);
 }
 void launch_ingest_normalised(const DeviceState& s, const float* d_x, int n, cudaStream_t st) {
     Mat9 k = {{1, 0, 0, 0, 1, 0, 0, 0, 1}};
@@ -269,7 +284,8 @@ __global__ void __launch_bounds__(256) choose_pose_vote_kernel(DeviceState s, fl
     __syncthreads();
     int local[4] = {0, 0, 0, 0};
     const float4* corr = s.corr + (size_t)b * s.n_stride;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < s.n; i += gridDim.x * blockDim.x) {
+    const int n = pair_n(s, b);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         float4 p = corr[i];
         if (epipolar_d(s.metric, sE, p.x, p.y, p.z, p.w, -thr) >= 0.0f) continue;
 #pragma unroll
@@ -338,7 +354,9 @@ constexpr int TRI_THREADS = SFMB200_TRI_THREADS;
 #ifndef SFMB200_TRI_MINB
 #define SFMB200_TRI_MINB 8      // resident CTAs per SM the kernel is compiled for (<= 64 registers at 128 threads)
 #endif
-template <int PTS, bool INLIERS_ONLY>
+// RAGGED: per-pair counts.  A compile-time case so that the uniform kernel keeps its bound in the constant bank: at the
+// 64-register cap one more live register spills.
+template <int PTS, bool INLIERS_ONLY, bool RAGGED>
 __global__ void __launch_bounds__(TRI_THREADS, SFMB200_TRI_MINB) triangulate_kernel(DeviceState s, float thr) {
     static_assert(PTS == 1 || PTS == 2, "one point per thread, or two in packed f32x2 arithmetic");
     pdl_wait();
@@ -361,7 +379,7 @@ __global__ void __launch_bounds__(TRI_THREADS, SFMB200_TRI_MINB) triangulate_ker
     // persistent over the pair's points: grid.x CTAs stride through them, the next points are in flight while the current
     // ones are solved (the loads are the only long-latency operation), the pose stays in registers
     constexpr int CHUNK = TRI_THREADS * PTS;
-    const int step = gridDim.x * CHUNK, n = s.n;
+    const int step = gridDim.x * CHUNK, n = RAGGED ? s.n_pair[b] : s.n;
     const float4* corr = s.corr + (size_t)b * s.n_stride;
     float* out = s.points + (size_t)b * 4 * s.n_stride;
     const float4 zero4 = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
@@ -436,7 +454,7 @@ template <bool INLIERS_ONLY>
 __global__ void __launch_bounds__(TRI_THREADS, SFMB200_TRI_MINB) triangulate_pairs_kernel(DeviceState s, float thr) {
     pdl_wait();
     const int b = blockIdx.y;
-    const int n = s.n, pairs = (n + 1) >> 1;            // an odd last point rides alone in the last pair (its twin is a copy)
+    const int n = pair_n(s, b), pairs = (n + 1) >> 1;            // an odd last point rides alone in the last pair (its twin is a copy)
     const float4* corr = s.corr + (size_t)b * s.n_stride;
     float* out = s.points + (size_t)b * 4 * s.n_stride;
     int j = blockIdx.x * TRI_THREADS + threadIdx.x;
@@ -522,10 +540,15 @@ void launch_triangulate(const DeviceState& s, int inliers_only, float thr, cudaS
     int gx = (s.n + CHUNK - 1) / CHUNK;
     if (gx > cap) gx = cap;      // (a grid of only-resident CTAs with equal shares was measured: 10.5 vs 9.8 us at 1M, 127 vs 121 us at 16M points)
     dim3 grid(gx, s.B);
-    if (inliers_only)
-        launch_dep(triangulate_kernel<SFMB200_TRI_PTS, true>, grid, dim3(TRI_THREADS), 0, st, s, thr);
+    const bool ragged = s.n_pair != nullptr;
+    if (inliers_only && ragged)
+        launch_dep(triangulate_kernel<SFMB200_TRI_PTS, true, true>, grid, dim3(TRI_THREADS), 0, st, s, thr);
+    else if (inliers_only)
+        launch_dep(triangulate_kernel<SFMB200_TRI_PTS, true, false>, grid, dim3(TRI_THREADS), 0, st, s, thr);
+    else if (ragged)
+        launch_dep(triangulate_kernel<SFMB200_TRI_PTS, false, true>, grid, dim3(TRI_THREADS), 0, st, s, thr);
     else
-        launch_dep(triangulate_kernel<SFMB200_TRI_PTS, false>, grid, dim3(TRI_THREADS), 0, st, s, thr);
+        launch_dep(triangulate_kernel<SFMB200_TRI_PTS, false, false>, grid, dim3(TRI_THREADS), 0, st, s, thr);
 #endif
 }
 
@@ -535,7 +558,7 @@ void launch_triangulate(const DeviceState& s, int inliers_only, float thr, cudaS
 // copyBoidsToVBO (sfm.cu:374-383, kernels.h:471-495): 4xN SoA -> Nx4 AoS, colour = 1.
 __global__ void vbo_kernel(DeviceState s, int pair, float4* pos, float4* col, float scale) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= s.n) return;
+    if (i >= pair_n(s, pair)) return;
     const float* in = s.points + (size_t)pair * 4 * s.n_stride;
     if (pos) pos[i] = make_float4(in[i] * scale, in[(size_t)s.n_stride + i] * scale, in[(size_t)2 * s.n_stride + i] * scale, 1.0f);
     if (col) col[i] = make_float4(1.0f, 1.0f, 1.0f, 1.0f);
@@ -546,7 +569,7 @@ __global__ void vbo_kernel(DeviceState s, int pair, float4* pos, float4* col, fl
 __global__ void vbo_colour_kernel(DeviceState s, int pair, float4* pos, float4* col, float scale, int mode, float thr,
                                   float z_near, float z_far) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= s.n) return;
+    if (i >= pair_n(s, pair)) return;
     const float* in = s.points + (size_t)pair * 4 * s.n_stride;
     const float X = in[i], Y = in[(size_t)s.n_stride + i], Z = in[(size_t)2 * s.n_stride + i];
     if (pos) pos[i] = make_float4(X * scale, Y * scale, Z * scale, 1.0f);
@@ -592,11 +615,12 @@ void launch_export_ecand(const DeviceState& s, int pair, int H, float* d_out, cu
 // X[image] as the reference stores it: 3xN row-major, rows x, y, 1 (sfm.cu:88-89).
 __global__ void export_X_kernel(DeviceState s, int pair, int image, float* out) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= s.n) return;
+    const int n = pair_n(s, pair);
+    if (i >= n) return;
     float4 p = s.corr[(size_t)pair * s.n_stride + i];
     out[i] = image == 0 ? p.x : p.z;
-    out[(size_t)s.n + i] = image == 0 ? p.y : p.w;
-    out[(size_t)2 * s.n + i] = 1.0f;
+    out[(size_t)n + i] = image == 0 ? p.y : p.w;
+    out[(size_t)2 * n + i] = 1.0f;
 }
 void launch_export_X(const DeviceState& s, int pair, int image, float* d_out, cudaStream_t st) {
     export_X_kernel<<<(s.n + 255) / 256, 256, 0, st>>>(s, pair, image, d_out);
@@ -606,7 +630,7 @@ void launch_export_X(const DeviceState& s, int pair, int image, float* d_out, cu
 // homography in s.E (thr = squared threshold)
 __global__ void inlier_mask_kernel(DeviceState s, int pair, float thr, int model, unsigned char* mask) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= s.n) return;
+    if (i >= pair_n(s, pair)) return;
     float e[9];
 #pragma unroll
     for (int k = 0; k < 9; k++) e[k] = s.E[(size_t)pair * 9 + k];

@@ -35,7 +35,7 @@ hypgen_kernel(DeviceState s, const int32_t* __restrict__ d_idx, long long idx_pa
     const int32_t* rows = d_idx ? d_idx + (size_t)b * idx_pair_stride : nullptr;
     Corr pts[8];
     float E[9];
-    bool ok = load_sample(corr, s.n, rows, seed + 0x632BE59BD9B4E019ull * (unsigned long long)b,
+    bool ok = load_sample(corr, pair_n(s, b), rows, seed + 0x632BE59BD9B4E019ull * (unsigned long long)b,
                           (long long)h_offset + (live ? j : 0), pts, s.sampler);
     if (SOLVER == 0) solve_hypothesis<SYNC>(pts, E);
     else if (SOLVER == 1) solve_hypothesis_projector(pts, E);
@@ -76,7 +76,8 @@ __global__ void regen_best_kernel(DeviceState s, const int32_t* __restrict__ d_i
     const int32_t* rows = d_idx ? d_idx + (size_t)b * idx_pair_stride : nullptr;
     Corr pts[8];
     float E[9];
-    bool ok = load_sample(corr, s.n, rows, seed + 0x632BE59BD9B4E019ull * (unsigned long long)b, (long long)hg, pts, s.sampler);
+    bool ok = load_sample(corr, pair_n(s, b), rows, seed + 0x632BE59BD9B4E019ull * (unsigned long long)b, (long long)hg, pts,
+                          s.sampler);
     if (solver == 0) solve_hypothesis<0>(pts, E);      // same code path as hypgen_kernel: bit-identical E
     else if (solver == 1) solve_hypothesis_projector(pts, E);
     else solve_homography(pts, E);
@@ -117,7 +118,7 @@ __global__ void adaptive_decide_kernel(DeviceState s, int* adapt, int round_begi
         }
         s.best_idx[b] = (int)hg;
         s.best_count[b] = cnt;
-        double w = (double)cnt / (double)s.n;
+        double w = (double)cnt / (double)pair_n(s, b);
         double w2 = w * w, w4 = w2 * w2, w8 = w4 * w4;
         bool ok = w8 >= 1.0 || (w8 > 0.0 && (double)done_after >= log1mp / log1p(-w8));
         mine += ok ? 0 : 1;

@@ -33,7 +33,7 @@ struct DeviceState {
                         // groups of 8 (the reference's scheme, sfm.cu:95-104)
     int n_max;          // capacity: correspondences per pair
     int h_max;          // capacity: hypotheses per pair (local slice)
-    int n;              // current correspondences per pair
+    int n;              // current correspondences per pair (per-pair-count mode: the largest count)
     int n_stride;       // points stride (n_max rounded up to SCORE_CHUNK)
     int h_stride;       // hypothesis stride (h_max rounded up to 1024)
     int tiles_max;
@@ -58,6 +58,22 @@ struct DeviceState {
     int* tri_count;     // [B] points triangulated in front of both cameras (diagnostic)
     int* vote;          // [B][8] cheirality votes of the four candidates + ticket (choose_pose_vote_kernel)
     int metric;         // inlier test of the essential-matrix model: 0 Sampson error (default), 1 symmetric epipolar distance
+    // Per-pair-count mode (the last ingest was *_ragged): pair b holds n_pair[b] correspondences and n is the largest
+    // of them (grid sizes).  nullptr on a uniform handle, where every pair holds n.  Kernels use pair_n().
+    const int* n_pair;             // [B]
+    const long long* grain_off;    // [B + 1] prefix sum of ceil(n_pair[b] / SCORE_GRAIN): the scoring work space
+};
+
+// Correspondences of pair b.
+__device__ __forceinline__ int pair_n(const DeviceState& s, int b) { return s.n_pair ? s.n_pair[b] : s.n; }
+
+// Correspondence counts of a batch as the score planner needs them: the largest (grains per tile of a uniform batch),
+// the sum (evaluations per hypothesis), the sum of ceil(count / SCORE_GRAIN) (the work space in grains per tile) and
+// whether the counts are per pair (which instantiation of the scoring kernel runs).
+struct PointCounts {
+    int B, n_max;
+    long long n_sum, grains;
+    bool ragged;
 };
 
 // Scratch of the local-optimisation (refit) stage, per pair.
@@ -137,18 +153,21 @@ void launch_ingest_sift(const DeviceState& s, const void* d_sift, int n, cudaStr
 void launch_ingest_sift_filtered(const DeviceState& s, const void* d_sift, int n, float min_score, float max_ambiguity,
                                  int* d_scratch, int* d_kept_index, cudaStream_t st);
 void launch_ingest_xy(const DeviceState& s, const float* d_px, int n, cudaStream_t st);
+// packed rows: pair b's s.n_pair[b] rows start at row d_row_off[b] of d_px
+void launch_ingest_xy_ragged(const DeviceState& s, const float* d_px, const int* d_row_off, cudaStream_t st);
 void launch_ingest_normalised(const DeviceState& s, const float* d_x, int n, cudaStream_t st);
 void launch_rescale_points(const DeviceState& s, cudaStream_t st);   // corr -> corr_s with s.pt_scale
 void launch_hypgen(const DeviceState& s, const int32_t* d_idx, long long idx_pair_stride, int H, int h_offset,
                    unsigned long long seed, int solver, cudaStream_t st, int keep_best = 0);
 void launch_adaptive_decide(const DeviceState& s, int* d_adapt, int round_begin, int done_after, double log1mp, int last,
                             cudaStream_t st);
-ScorePlan make_score_plan(int B, int n, int H, int variant_override, int sms);
+ScorePlan make_score_plan(const PointCounts& c, int H, int variant_override, int sms);
 int score_num_variants();
-void launch_score(const DeviceState& s, const ScorePlan& plan, int H, int h_offset, float thr, cudaStream_t st);
+// h_n_pair: host copy of s.n_pair (nullptr on a uniform handle); the constant-bank variant sizes its launches with it
+void launch_score(const DeviceState& s, const ScorePlan& plan, int H, int h_offset, float thr, const int* h_n_pair, cudaStream_t st);
 void launch_score_homography(const DeviceState& s, ScorePlan& plan, int H, int h_offset, float thr2, cudaStream_t st);
-void launch_score_symmetric(const DeviceState& s, ScorePlan& plan, int H, int h_offset, float thr, cudaStream_t st);
-ScorePlan make_score_plan_homography(int B, int n, int H, int sms);
+void launch_score_symmetric(const DeviceState& s, ScorePlan& plan, int H, int h_offset, float thr, const int* h_n_pair, cudaStream_t st);
+ScorePlan make_score_plan_homography(const PointCounts& c, int H, int sms);
 void launch_select(const DeviceState& s, int h_offset, cudaStream_t st);
 void launch_regen_best(const DeviceState& s, const int32_t* d_idx, long long idx_pair_stride,
                        unsigned long long seed, int solver, cudaStream_t st);

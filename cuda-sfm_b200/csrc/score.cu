@@ -32,6 +32,7 @@
 #include <math.h>
 
 #include <mutex>
+#include <type_traits>
 
 #include "internal.cuh"
 #include "sampson.cuh"
@@ -91,26 +92,68 @@ __device__ __forceinline__ unsigned long long warp_max_u64(unsigned long long v)
 // ("stream-K" decomposition along the point axis), so there is no tail wave.
 // A CTA's share is a sequence of segments, each a contiguous point range of one
 // (pair, tile); segments are streamed chunk by chunk.
-struct ChunkWalk {
+// Per-pair counts (RAGGED): pair b owns units [T * goff[b], T * goff[b + 1]), tile-major inside; with equal counts that
+// is the uniform layout.  Shares cross pair boundaries like tile boundaries, so one large pair among small ones splits
+// over every CTA.  The pair of the first unit is found by a binary search over goff; after that a segment starts in the
+// same pair or the next one.  The uniform walk is the RAGGED = false case: it reads nothing but kernel parameters.
+struct RaggedCursor {
+    const long long* goff; // grain prefix (DeviceState::grain_off) and counts (DeviceState::n_pair)
+    const int* n_pair;
+    long long pair_lo, pair_hi;   // units of the current pair
+};
+struct UniformCursor {};
+template <bool RAGGED>
+struct ChunkWalk : std::conditional_t<RAGGED, RaggedCursor, UniformCursor> {
     long long u, end;      // grain cursor / end of this CTA's share
-    int n_units, n, T;     // grains per tile, points per pair, tiles per pair
+    int n_units, n, T;     // grains per tile, points of the current pair, tiles per pair
     int b, t, p0, cnt;     // current chunk: pair, tile, first point, points
     int seg_p0, seg_pts;   // current segment: first point, total points
     int left;              // points of the segment not yet handed out
     bool seg_first, seg_last;
-    __device__ __forceinline__ void init(long long u0, long long u1, int n_units_, int n_, int T_) {
+    __device__ __forceinline__ void set_pair(int b_) {
+        b = b_;
+        this->pair_lo = (long long)T * this->goff[b];
+        this->pair_hi = (long long)T * this->goff[b + 1];
+        n_units = (int)(this->goff[b + 1] - this->goff[b]);
+        n = this->n_pair[b];
+    }
+    __device__ __forceinline__ void init(long long u0, long long u1, int n_units_, int n_, int T_, int B,
+                                         const long long* goff_, const int* n_pair_) {
         u = u0; end = u1; n_units = n_units_; n = n_; T = T_;
         left = 0; cnt = 0; p0 = 0;
+        if constexpr (RAGGED) {
+            this->goff = goff_;
+            this->n_pair = n_pair_;
+            if (u0 < u1) {
+                int lo = 0, hi = B - 1;          // the last pair whose first unit is <= u0
+                while (lo < hi) {
+                    const int mid = (lo + hi + 1) >> 1;
+                    if ((long long)T * goff_[mid] <= u0) lo = mid; else hi = mid - 1;
+                }
+                set_pair(lo);
+            }
+        }
     }
     __device__ __forceinline__ bool next() {
         if (left == 0) {
             if (u >= end) return false;
-            long long bt = u / n_units;
-            int pu = (int)(u - bt * n_units);
+            long long bt = 0;
+            int pu;
+            if constexpr (RAGGED) {
+                while (u >= this->pair_hi) set_pair(b + 1);
+                const long long rel = u - this->pair_lo;
+                t = (int)(rel / n_units);
+                pu = (int)(rel - (long long)t * n_units);
+            } else {
+                bt = u / n_units;
+                pu = (int)(u - bt * n_units);
+            }
             long long seg_units = end - u;
             if (seg_units > n_units - pu) seg_units = n_units - pu;
-            b = (int)(bt / T);
-            t = (int)(bt - (long long)b * T);
+            if constexpr (!RAGGED) {
+                b = (int)(bt / T);
+                t = (int)(bt - (long long)b * T);
+            }
             seg_p0 = pu * SCORE_GRAIN;
             int p1 = (pu + (int)seg_units) * SCORE_GRAIN;
             if (p1 > n) p1 = n;
@@ -139,7 +182,7 @@ struct ChunkWalk {
 // every thread of the CTA.
 // `full`: this CTA saw every point of the tile.  Otherwise the tile's ticket counter advances by
 // `inc` and the CTA that brings it to `total` completes the tile (TMA path: points processed out
-// of n; constant-bank path: CTA arrivals out of the number the host scheduled for the tile).
+// of the pair's count; constant-bank path: CTA arrivals out of the number the host scheduled for the tile).
 template <int HPT, int THREADS>
 __device__ __forceinline__ void segment_epilogue(const DeviceState& s, int b, int t, int H, int h_offset,
                                                  const unsigned int* cnt, bool full, int inc, int total,
@@ -210,7 +253,7 @@ struct ChunkDesc {
     int seg_pts;       // points of the whole segment (valid when seg_last)
 };
 
-template <int HPT, bool PACKED, int THREADS, int MINB, int MODEL>
+template <int HPT, bool PACKED, int THREADS, int MINB, int MODEL, bool RAGGED = false>
 __global__ void __launch_bounds__(THREADS, MINB)
 score_kernel(DeviceState s, int H, int h_offset, int T, long long total_units, int n_units, float thr) {
     constexpr int HPC = HPT * THREADS;
@@ -220,8 +263,9 @@ score_kernel(DeviceState s, int H, int h_offset, int T, long long total_units, i
     __shared__ __align__(128) float4 buf[2][SCORE_CHUNK];
     __shared__ __align__(8) uint64_t full[2];
     __shared__ __align__(16) ChunkDesc desc[2];
-    __shared__ ChunkWalk walk;          // producer state lives here, not in loop-carried registers:
+    __shared__ ChunkWalk<RAGGED> walk;  // producer state lives here, not in loop-carried registers:
                                         // the FFMA stream needs every register for operand reuse
+    __shared__ int desc_n[2];           // RAGGED: points of the pair of desc[]
     __shared__ unsigned long long red[THREADS / 32];
     __shared__ int s_last;
 
@@ -233,8 +277,9 @@ score_kernel(DeviceState s, int H, int h_offset, int T, long long total_units, i
         mbar_init(&full[0], 1);
         mbar_init(&full[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        ChunkWalk w;
-        w.init(total_units * blockIdx.x / gridDim.x, total_units * (blockIdx.x + 1) / gridDim.x, n_units, s.n, T);
+        ChunkWalk<RAGGED> w;
+        w.init(total_units * blockIdx.x / gridDim.x, total_units * (blockIdx.x + 1) / gridDim.x, n_units, s.n, T, s.B,
+               s.grain_off, s.n_pair);
         walk = w;
     }
     __syncthreads();
@@ -242,11 +287,12 @@ score_kernel(DeviceState s, int H, int h_offset, int T, long long total_units, i
     // Producer step (thread 0): advance the walk, publish the descriptor of the
     // next chunk and start its TMA; an empty descriptor + plain arrive ends the loop.
     auto produce = [&](int stage) {
-        ChunkWalk w = walk;
+        ChunkWalk<RAGGED> w = walk;
         bool more = w.next();
         walk = w;
         ChunkDesc d;
         d.b = w.b; d.t = w.t; d.seg_pts = w.seg_pts;
+        if constexpr (RAGGED) desc_n[stage] = w.n;
         d.cnt_flags = more ? (w.cnt | (w.seg_first ? (1 << 30) : 0) | (w.seg_last ? (1 << 31) : 0)) : 0;
         desc[stage] = d;
         if (more) {
@@ -323,7 +369,10 @@ score_kernel(DeviceState s, int H, int h_offset, int T, long long total_units, i
         if (d.cnt_flags >= 0) continue;   // bit 31 clear: segment continues
 
         // ---- end of a segment: counts + fused arg-max for (pair b, tile t) ----
-        segment_epilogue<HPT, THREADS>(s, d.b, d.t, H, h_offset, cnt, d.seg_pts == s.n, d.seg_pts, s.n, red, &s_last);
+        // (read here, not with d: the pair's count need not stay in a register across the point loop; the producer
+        // rewrites desc_n[k & 1] only after the barrier inside the epilogue)
+        const int n_b = RAGGED ? desc_n[k & 1] : s.n;
+        segment_epilogue<HPT, THREADS>(s, d.b, d.t, H, h_offset, cnt, d.seg_pts == n_b, d.seg_pts, n_b, red, &s_last);
     }
 }
 
@@ -430,25 +479,30 @@ struct ConstBankGuard {
 static ConstBankGuard g_const;
 
 template <int MODEL>
-static void launch_score_const(const DeviceState& s, const ScorePlan& plan, int H, int h_offset, float thr, cudaStream_t st) {
+static void launch_score_const(const DeviceState& s, const ScorePlan& plan, int H, int h_offset, float thr, const int* h_n_pair,
+                               cudaStream_t st) {
     int dev = 0;
     cudaGetDevice(&dev);
     dev &= 63;
     std::lock_guard<std::mutex> lock(g_const.mu);
     if (!g_const.last_use[dev]) cudaEventCreateWithFlags(&g_const.last_use[dev], cudaEventDisableTiming);
-    const int batches = (s.n + CONST_PTS - 1) / CONST_PTS;
-    const int per = ((s.n + batches - 1) / batches + 15) / 16 * 16;      // even batches
-    // pass 1: the split of every batch, and with it the CTA arrivals each tile will see in total
-    int arrivals = 0;
-    for (int off = 0; off < s.n; off += per) {
-        const int cnt = s.n - off < per ? s.n - off : per;
-        const int splits = const_splits(plan.tiles, cnt, plan.ctas);        // plan.ctas = resident CTA slots
-        const int chunk = (cnt + splits - 1) / splits;
-        arrivals += (cnt + chunk - 1) / chunk;
-    }
-    for (int b = 0; b < s.B; b++)
-        for (int off = 0; off < s.n; off += per) {
-            const int cnt = s.n - off < per ? s.n - off : per;
+    int n = -1, per = 0, arrivals = 0;
+    for (int b = 0; b < s.B; b++) {
+        const int nb = h_n_pair ? h_n_pair[b] : s.n;
+        if (nb != n) {      // a new count: batches of the pair and the CTA arrivals each of its tiles will see in total
+            n = nb;
+            const int batches = (n + CONST_PTS - 1) / CONST_PTS;
+            per = ((n + batches - 1) / batches + 15) / 16 * 16;      // even batches
+            arrivals = 0;
+            for (int off = 0; off < n; off += per) {
+                const int cnt = n - off < per ? n - off : per;
+                const int splits = const_splits(plan.tiles, cnt, plan.ctas);        // plan.ctas = resident CTA slots
+                const int chunk = (cnt + splits - 1) / splits;
+                arrivals += (cnt + chunk - 1) / chunk;
+            }
+        }
+        for (int off = 0; off < n; off += per) {
+            const int cnt = n - off < per ? n - off : per;
             const int splits = const_splits(plan.tiles, cnt, plan.ctas);
             const int chunk = (cnt + splits - 1) / splits;
             const int real_splits = (cnt + chunk - 1) / chunk;
@@ -460,6 +514,7 @@ static void launch_score_const(const DeviceState& s, const ScorePlan& plan, int 
                 <<<dim3(plan.tiles, real_splits), CONST_THREADS, 0, st>>>(s, b, chunk, last_np, arrivals, H, h_offset, thr);
             cudaEventRecord(g_const.last_use[dev], st);
         }
+    }
 }
 
 // Kernel family.  Register-bank bandwidth is what bounds the FP32 pipe here: an
@@ -493,12 +548,16 @@ constexpr int kNumVariants = sizeof(kVariants) / sizeof(kVariants[0]);
 template <int HPT, bool PACKED, int THREADS, int MINB>
 static void launch_one(const DeviceState& s, int ctas, int H, int h_offset, int T, long long units, int n_units, float thr,
                        cudaStream_t st) {
-    launch_dep(score_kernel<HPT, PACKED, THREADS, MINB, 0>, dim3(ctas), dim3(THREADS), 0, st, s, H, h_offset, T, units, n_units, thr);
+    if (s.n_pair)
+        launch_dep(score_kernel<HPT, PACKED, THREADS, MINB, 0, true>, dim3(ctas), dim3(THREADS), 0, st, s, H, h_offset, T, units, n_units, thr);
+    else
+        launch_dep(score_kernel<HPT, PACKED, THREADS, MINB, 0>, dim3(ctas), dim3(THREADS), 0, st, s, H, h_offset, T, units, n_units, thr);
 }
 template <int HPT, bool PACKED, int THREADS, int MINB>
-static int occupancy_one() {
+static int occupancy_one(bool ragged) {
     int n = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, score_kernel<HPT, PACKED, THREADS, MINB, 0>, THREADS, 0);
+    if (ragged) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, score_kernel<HPT, PACKED, THREADS, MINB, 0, true>, THREADS, 0);
+    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, score_kernel<HPT, PACKED, THREADS, MINB, 0>, THREADS, 0);
     return n > 0 ? n : 1;
 }
 #define SFM_FOR_VARIANT(v, CALL)                     \
@@ -516,24 +575,25 @@ static int occupancy_one() {
         default: CALL(2, false, 128, 1); break;      \
     }
 
-static int variant_occupancy(int v) {
-    static int cache[kNumVariants] = {0};
-    if (cache[v] == 0 && v == kConstVariant) {
+static int variant_occupancy(int v, bool ragged) {
+    static int cache[2][kNumVariants] = {};
+    int& c = cache[ragged ? 1 : 0][v];
+    if (c == 0 && v == kConstVariant) {
         int n = 0;
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, score_const_kernel<CONST_HPT, CONST_THREADS, CONST_MINB, 0>, CONST_THREADS, 0);
-        cache[v] = n > 0 ? n : 1;
+        c = n > 0 ? n : 1;
     }
-    if (cache[v] == 0) {
-#define SFM_OCC(h, p, t, m) cache[v] = occupancy_one<h, p, t, m>()
+    if (c == 0) {
+#define SFM_OCC(h, p, t, m) c = occupancy_one<h, p, t, m>(ragged)
         SFM_FOR_VARIANT(v, SFM_OCC)
 #undef SFM_OCC
     }
-    return cache[v];
+    return c;
 }
 
 int score_num_variants() { return kNumVariants; }
 
-ScorePlan make_score_plan(int B, int n, int H, int variant_override, int sms) {
+ScorePlan make_score_plan(const PointCounts& c, int H, int variant_override, int sms) {
     ScorePlan p;
     if (variant_override >= 0 && variant_override < kNumVariants) {
         p.variant = variant_override;
@@ -543,7 +603,7 @@ ScorePlan make_score_plan(int B, int n, int H, int variant_override, int sms) {
         // kernel is latency- rather than throughput-bound and the 512-hypothesis tile (6), below ~3e7 the 256-hypothesis
         // scalar tile (9) win by up to 24 %.  The constant-bank kernel (variant 10) is never chosen automatically: see the
         // note above score_const_kernel.
-        const double W = (double)B * (double)n * (double)H;       // evaluations per launch
+        const double W = (double)c.n_sum * (double)H;       // evaluations per launch
         if (H >= 1536) p.variant = W >= 1.2e8 ? 4 : 6;
         else if (H >= 768) p.variant = W >= 2e8 ? 1 : (W >= 3e7 ? 6 : 9);
         else p.variant = W >= 3e7 ? 6 : 9;
@@ -553,9 +613,9 @@ ScorePlan make_score_plan(int B, int n, int H, int variant_override, int sms) {
     p.tiles = (H + p.hyp_per_cta - 1) / p.hyp_per_cta;
     if (p.tiles < 1) p.tiles = 1;
     if (sms < 1) sms = 148;          // the handle caches the SM count of ITS device at create (api.cu)
-    p.n_units = (n + SCORE_GRAIN - 1) / SCORE_GRAIN;
-    p.total_units = (long long)B * p.tiles * p.n_units;
-    long long ctas = (long long)sms * variant_occupancy(p.variant);   // persistent: all CTAs co-resident
+    p.n_units = (c.n_max + SCORE_GRAIN - 1) / SCORE_GRAIN;      // used by the uniform walk only
+    p.total_units = (long long)p.tiles * c.grains;
+    long long ctas = (long long)sms * variant_occupancy(p.variant, c.ragged);   // persistent: all CTAs co-resident
     if (p.variant != kConstVariant && ctas > p.total_units) ctas = p.total_units;   // const path: ctas = resident slots
     if (ctas < 1) ctas = 1;
     p.ctas = (int)ctas;
@@ -564,25 +624,30 @@ ScorePlan make_score_plan(int B, int n, int H, int variant_override, int sms) {
 
 // Homography model: the same kernel with the transfer-error test; three tile sizes are enough
 // (thr here is the SQUARED pixel / coordinate threshold).
-ScorePlan make_score_plan_homography(int B, int n, int H, int sms) {
+ScorePlan make_score_plan_homography(const PointCounts& c, int H, int sms) {
 #ifdef SFMB200_HOMOG_PLAN_BY_H      // the rule before the sweep (A/B)
-    return make_score_plan(B, n, H, H >= 1536 ? 4 : (H >= 384 ? 6 : 9), sms);     // tiles of 2048 / 512 / 256 hypotheses
+    return make_score_plan(c, H, H >= 1536 ? 4 : (H >= 384 ? 6 : 9), sms);     // tiles of 2048 / 512 / 256 hypotheses
 #else
-    const double W = (double)B * (double)n * (double)H;      // same reading as make_score_plan: small launches are latency-bound
-    return make_score_plan(B, n, H, H >= 1536 ? (W >= 1.2e8 ? 4 : 6) : (W >= 3e7 ? 6 : 9), sms);
+    const double W = (double)c.n_sum * (double)H;      // same reading as make_score_plan: small launches are latency-bound
+    return make_score_plan(c, H, H >= 1536 ? (W >= 1.2e8 ? 4 : 6) : (W >= 3e7 ? 6 : 9), sms);
 #endif
 }
 // The other two models (homography transfer error; symmetric epipolar distance) in the three tile sizes of
 // make_score_plan_homography.
 template <int MODEL>
-static void launch_score_model(const DeviceState& s, ScorePlan& plan, int H, int h_offset, float thr, cudaStream_t st) {
+static void launch_score_model(const DeviceState& s, ScorePlan& plan, int H, int h_offset, float thr, const int* h_n_pair,
+                               cudaStream_t st) {
     const int v = plan.variant;
     if (v == kConstVariant) {
-        launch_score_const<MODEL>(s, plan, H, h_offset, thr, st);
+        launch_score_const<MODEL>(s, plan, H, h_offset, thr, h_n_pair, st);
         return;
     }
     const bool big = kVariants[v].hpt * kVariants[v].threads >= 2048, mid = kVariants[v].hpt * kVariants[v].threads >= 512;
-    if (big) {
+    if (s.n_pair) {
+        if (big) score_kernel<8, true, 256, 1, MODEL, true><<<plan.ctas, 256, 0, st>>>(s, H, h_offset, plan.tiles, plan.total_units, plan.n_units, thr);
+        else if (mid) score_kernel<4, true, 128, 1, MODEL, true><<<plan.ctas, 128, 0, st>>>(s, H, h_offset, plan.tiles, plan.total_units, plan.n_units, thr);
+        else score_kernel<2, false, 128, 1, MODEL, true><<<plan.ctas, 128, 0, st>>>(s, H, h_offset, plan.tiles, plan.total_units, plan.n_units, thr);
+    } else if (big) {
         score_kernel<8, true, 256, 1, MODEL><<<plan.ctas, 256, 0, st>>>(s, H, h_offset, plan.tiles, plan.total_units, plan.n_units, thr);
     } else if (mid) {
         score_kernel<4, true, 128, 1, MODEL><<<plan.ctas, 128, 0, st>>>(s, H, h_offset, plan.tiles, plan.total_units, plan.n_units, thr);
@@ -591,15 +656,17 @@ static void launch_score_model(const DeviceState& s, ScorePlan& plan, int H, int
     }
 }
 void launch_score_homography(const DeviceState& s, ScorePlan& plan, int H, int h_offset, float thr2, cudaStream_t st) {
-    launch_score_model<1>(s, plan, H, h_offset, thr2, st);
+    launch_score_model<1>(s, plan, H, h_offset, thr2, nullptr, st);
 }
-void launch_score_symmetric(const DeviceState& s, ScorePlan& plan, int H, int h_offset, float thr, cudaStream_t st) {
-    launch_score_model<2>(s, plan, H, h_offset, thr, st);
+void launch_score_symmetric(const DeviceState& s, ScorePlan& plan, int H, int h_offset, float thr, const int* h_n_pair,
+                            cudaStream_t st) {
+    launch_score_model<2>(s, plan, H, h_offset, thr, h_n_pair, st);
 }
 
-void launch_score(const DeviceState& s, const ScorePlan& plan, int H, int h_offset, float thr, cudaStream_t st) {
+void launch_score(const DeviceState& s, const ScorePlan& plan, int H, int h_offset, float thr, const int* h_n_pair,
+                  cudaStream_t st) {
     if (plan.variant == kConstVariant) {
-        launch_score_const<0>(s, plan, H, h_offset, thr, st);
+        launch_score_const<0>(s, plan, H, h_offset, thr, h_n_pair, st);
         return;
     }
 #define SFM_LAUNCH(h, p, t, m) launch_one<h, p, t, m>(s, plan.ctas, H, h_offset, plan.tiles, plan.total_units, plan.n_units, thr, st)

@@ -48,8 +48,51 @@ def _hptr(a: np.ndarray, dtype=None, shape: tuple | None = None) -> C.c_void_p:
     return C.c_void_p(a.ctypes.data)
 
 
+def pack_ragged(parts):
+    """Per-pair (count_b, 4) rows -> (packed rows [sum count_b][4], offsets int32 [pairs + 1]), the layout of the
+    *_ragged entry points.  numpy arrays stay numpy (float32); torch tensors are concatenated by torch (same device)."""
+    if len(parts) == 0:
+        raise ValueError("no pairs")
+    counts = [int(p.shape[0]) for p in parts]
+    offsets = np.zeros(len(parts) + 1, np.int32)
+    offsets[1:] = np.cumsum(counts)
+    if hasattr(parts[0], "is_cuda"):
+        torch = _torch()
+        packed = torch.cat([p.reshape(-1, 4).to(torch.float32) for p in parts]).contiguous()
+    else:
+        packed = np.ascontiguousarray(np.concatenate([np.asarray(p, np.float32).reshape(-1, 4) for p in parts]))
+    return packed, offsets
+
+
+def unpack_ragged(packed, offsets) -> list:
+    """Inverse of pack_ragged: the views packed[offsets[b]:offsets[b + 1]].  For a packed [4][count_b] SoA output (points
+    of run_host_ragged) pass it viewed as rows of 4 floats and reshape each part to (4, -1)."""
+    return [packed[int(offsets[b]):int(offsets[b + 1])] for b in range(len(offsets) - 1)]
+
+
+def check_offsets(offsets, pairs: int, max_points: int, rows: int | None = None) -> np.ndarray:
+    """The C ABI's checks of a ragged batch's offsets, done before any call: int32 [pairs + 1], offsets[0] == 0, every
+    count in [8, max_points] and, when given, rows == offsets[pairs].  Returns the offsets as a C-contiguous int32 array."""
+    o = np.asarray(offsets)
+    if o.ndim != 1 or o.shape[0] != pairs + 1:
+        raise ValueError(f"offsets must have pairs + 1 = {pairs + 1} entries, got shape {o.shape}")
+    if not np.issubdtype(o.dtype, np.integer):
+        raise TypeError(f"offsets must be integers, got {o.dtype}")
+    o = o.astype(np.int64)
+    if o[0] != 0:
+        raise ValueError("offsets[0] must be 0")
+    c = np.diff(o)
+    if np.any(c < 0):
+        raise ValueError("offsets must not decrease")
+    if np.any(c < 8) or np.any(c > max_points):
+        raise ValueError(f"every count offsets[b+1] - offsets[b] must be in [8, max_points={max_points}]")
+    if rows is not None and rows != o[-1]:
+        raise ValueError(f"the packed input has {rows} rows, offsets[-1] = {o[-1]}")
+    return np.ascontiguousarray(o.astype(np.int32))
+
+
 class BatchedPairs:
-    """A handle over `pairs` image pairs with n correspondences each."""
+    """A handle over `pairs` image pairs with n correspondences each, or count_b for pair b (the *_ragged methods)."""
 
     def __init__(self, K, Kinv, pairs: int, max_points: int, max_hypotheses: int, lib: Lib | None = None):
         self.lib = lib or load_library()
@@ -58,6 +101,7 @@ class BatchedPairs:
         self.pairs, self.max_points, self.max_hypotheses = pairs, max_points, max_hypotheses
         self.n = 0
         self.H = 0
+        self.counts = None        # per-pair counts after a *_ragged ingest, None while every pair holds n
         h = C.c_void_p()
         fp = C.POINTER(C.c_float)
         self.lib.call("sfmb200_create", self.K.ctypes.data_as(fp), self.Kinv.ctypes.data_as(fp), pairs, max_points,
@@ -93,7 +137,7 @@ class BatchedPairs:
     # ---- ingest ----
     def set_points_sift(self, d_sift, n: int):
         self.lib.call("sfmb200_set_points_sift", self._h, _dptr(d_sift), n)
-        self.n = n
+        self.n, self.counts = n, None
 
     def set_points_sift_filtered(self, d_sift, n: int, min_score: float, max_ambiguity: float, d_kept_index=None) -> int:
         kept = C.c_int32(0)
@@ -101,25 +145,90 @@ class BatchedPairs:
             self.lib.call("sfmb200_set_points_sift_filtered", self._h, _dptr(d_sift), n, C.c_float(min_score),
                           C.c_float(max_ambiguity), _dptr(d_kept_index), C.byref(kept))
         finally:
-            self.n = kept.value
+            self.n, self.counts = kept.value, None
         return kept.value
 
     def set_points_xy(self, d_px, n: int | None = None):
         n = n if n is not None else d_px.shape[-2]
         self.lib.call("sfmb200_set_points_xy", self._h, _dptr(d_px, "float32", self.pairs * n * 4), n)
-        self.n = n
+        self.n, self.counts = n, None
 
     def set_points_xy_host(self, h_px: np.ndarray):
         h_px = np.ascontiguousarray(h_px, dtype=np.float32)
         n = h_px.shape[-2]
         self.lib.call("sfmb200_set_points_xy_host", self._h, _hptr(h_px), n)
         self.synchronize()   # h_px may be pageable and die with the caller
-        self.n = n
+        self.n, self.counts = n, None
 
     def set_points_normalised(self, d_x, n: int | None = None):
         n = n if n is not None else d_x.shape[-2]
         self.lib.call("sfmb200_set_points_normalised", self._h, _dptr(d_x, "float32", self.pairs * n * 4), n)
-        self.n = n
+        self.n, self.counts = n, None
+
+    # ---- batches with a count per pair ----
+    def _ragged(self, px, offsets, device: bool):
+        """(packed rows, offsets) of a ragged input: a list of per-pair (count_b, 4) arrays / tensors, or packed rows with
+        their offsets.  device: a contiguous float32 CUDA tensor; else a C-contiguous float32 numpy array (a pinned one
+        is passed through untouched)."""
+        if offsets is None:
+            if not isinstance(px, (list, tuple)):
+                raise ValueError("pass a list of per-pair (count_b, 4) arrays, or packed rows with offsets")
+            px, offsets = pack_ragged(px)
+        torch = _torch() if device else None
+        if device:
+            if not hasattr(px, "is_cuda"):
+                px = torch.from_numpy(np.ascontiguousarray(px, dtype=np.float32))
+            px = px.to(device="cuda", dtype=torch.float32).contiguous()
+        elif not (isinstance(px, np.ndarray) and px.dtype == np.float32 and px.flags["C_CONTIGUOUS"]):
+            px = np.ascontiguousarray(px.cpu().numpy() if hasattr(px, "is_cuda") else px, dtype=np.float32)
+        if px.shape[-1] != 4 or px.ndim != 2:
+            raise ValueError(f"packed rows must be [rows][4], got {tuple(px.shape)}")
+        offsets = check_offsets(offsets, self.pairs, self.max_points, int(px.shape[0]))
+        return px, offsets
+
+    def _set_counts(self, offsets: np.ndarray):
+        self.counts = np.diff(offsets).astype(np.int32)
+        self.n = int(self.counts.max())
+
+    def set_points_xy_ragged(self, px, offsets=None):
+        """Pixel correspondences with a count per pair (include/sfmb200.h: sfmb200_set_points_xy_ragged)."""
+        px, offsets = self._ragged(px, offsets, True)
+        self.lib.call("sfmb200_set_points_xy_ragged", self._h, _dptr(px), _hptr(offsets))
+        self._set_counts(offsets)
+
+    def run_device_ragged(self, px, H: int, seed: int = 0, thr: float = 1e-6, offsets=None):
+        px, offsets = self._ragged(px, offsets, True)
+        self.lib.call("sfmb200_run_device_ragged", self._h, _dptr(px), _hptr(offsets), H, C.c_uint64(seed), C.c_float(thr))
+        self._set_counts(offsets)
+        self.H = H
+
+    def run_host_ragged(self, px, H: int, seed: int = 0, thr: float = 1e-6, offsets=None, want_points: bool = True) -> dict:
+        """Whole path from host pixel correspondences with a count per pair.  Returns E [pairs,9], P [pairs,16],
+        pose_index / inliers [pairs], points: a list of per-pair (4, count_b) arrays (views of points_packed, the
+        packed buffer the C ABI wrote) or None."""
+        px, offsets = self._ragged(px, offsets, False)
+        B = self.pairs
+        out = {"E": np.empty((B, 9), np.float32), "P": np.empty((B, 16), np.float32), "pose_index": np.empty(B, np.int32),
+               "inliers": np.empty(B, np.int32)}
+        packed = np.empty(4 * int(offsets[-1]), np.float32) if want_points else None
+        self.lib.call("sfmb200_run_host_ragged", self._h, _hptr(px), _hptr(offsets), H, C.c_uint64(seed), C.c_float(thr),
+                      _hptr(out["E"]), _hptr(out["P"]), _hptr(out["pose_index"]), _hptr(out["inliers"]),
+                      _hptr(packed) if want_points else C.c_void_p(0))
+        self._set_counts(offsets)
+        self.H = H
+        out["points_packed"] = packed
+        out["points"] = [p.reshape(4, -1) for p in unpack_ragged(packed.reshape(-1, 4), offsets)] if want_points else None
+        return out
+
+    def point_counts(self) -> np.ndarray:
+        """Correspondences per pair of the current points (n for every pair after a uniform ingest)."""
+        out = np.empty(self.pairs, np.int32)
+        self.lib.call("sfmb200_get_point_counts", self._h, _hptr(out))
+        return out
+
+    def _count(self, pair: int) -> int:
+        """Rows the per-pair getters return for `pair`."""
+        return int(self.counts[pair]) if self.counts is not None else self.n
 
     # ---- stages ----
     def estimate_e(self, H: int, seed: int = 0, thr: float = 1e-6, d_idx=None, H_total: int | None = None, h_begin: int = 0):
@@ -213,7 +322,7 @@ class BatchedPairs:
     def run_device(self, d_px, H: int, seed: int = 0, thr: float = 1e-6, n: int | None = None):
         n = n if n is not None else d_px.shape[-2]
         self.lib.call("sfmb200_run_device", self._h, _dptr(d_px, "float32", self.pairs * n * 4), n, H, C.c_uint64(seed), C.c_float(thr))
-        self.n, self.H = n, H
+        self.n, self.H, self.counts = n, H, None
 
     def _host_io(self, h_px: np.ndarray, want_points: bool, out: dict | None):
         """Validated host buffers of the e2e call: h_px float32 [pairs][n][4] (coerced like set_points_xy_host unless it
@@ -236,7 +345,7 @@ class BatchedPairs:
         """Whole path from host pixel correspondences to host results (the e2e call)."""
         h_px, n, out, ptrs = self._host_io(h_px, want_points, out)
         self.lib.call("sfmb200_run_host", self._h, _hptr(h_px), n, H, C.c_uint64(seed), C.c_float(thr), *ptrs)
-        self.n, self.H = n, H
+        self.n, self.H, self.counts = n, H, None
         return out
 
     def prepare_run_host(self, h_px: np.ndarray, H: int, seed: int = 0, thr: float = 1e-6, out: dict | None = None):
@@ -247,7 +356,7 @@ class BatchedPairs:
         args = (self._h, _hptr(h_px), n, H, C.c_uint64(seed), C.c_float(thr), *ptrs)
         fn = self.lib.raw("sfmb200_run_host")
         lib = self.lib
-        self.n, self.H = n, H
+        self.n, self.H, self.counts = n, H, None
 
         def call():
             rc = fn(*args)
@@ -283,13 +392,13 @@ class BatchedPairs:
         return out
 
     def get_points_host(self, pair: int = 0) -> np.ndarray:
-        out = np.empty((4, self.n), np.float32)
+        out = np.empty((4, self._count(pair)), np.float32)
         self.lib.call("sfmb200_get_points_host", self._h, pair, _hptr(out))
         return out
 
     def get_points(self, pair: int = 0):
         torch = _torch()
-        out = torch.empty((4, self.n), dtype=torch.float32, device="cuda")
+        out = torch.empty((4, self._count(pair)), dtype=torch.float32, device="cuda")
         self.lib.call("sfmb200_get_points", self._h, pair, _dptr(out))
         self.synchronize()
         return out
@@ -310,24 +419,26 @@ class BatchedPairs:
 
     def get_X(self, image: int, pair: int = 0):
         torch = _torch()
-        out = torch.empty((3, self.n), dtype=torch.float32, device="cuda")
+        out = torch.empty((3, self._count(pair)), dtype=torch.float32, device="cuda")
         self.lib.call("sfmb200_get_X", self._h, pair, image, _dptr(out))
         self.synchronize()
         return out
 
     def get_inlier_mask(self, pair: int = 0):
         torch = _torch()
-        out = torch.empty(self.n, dtype=torch.uint8, device="cuda")
+        out = torch.empty(self._count(pair), dtype=torch.uint8, device="cuda")
         self.lib.call("sfmb200_get_inlier_mask", self._h, pair, _dptr(out))
         self.synchronize()
         return out
 
     def copy_to_vbo(self, d_pos, d_col, pair: int = 0):
-        self.lib.call("sfmb200_copy_to_vbo", self._h, pair, _dptr(d_pos, "float32", 4 * self.n), _dptr(d_col, "float32", 4 * self.n))
+        n = self._count(pair)
+        self.lib.call("sfmb200_copy_to_vbo", self._h, pair, _dptr(d_pos, "float32", 4 * n), _dptr(d_col, "float32", 4 * n))
 
     def copy_to_vbo_coloured(self, d_pos, d_col, pair: int = 0, scale: float = 1.0, mode: int = 1, z_near: float = 0.0, z_far: float = 1.0):
         """mode 0 ones, 1 inlier green / outlier red, 2 depth ramp blue -> red between z_near and z_far."""
-        self.lib.call("sfmb200_copy_to_vbo_coloured", self._h, pair, _dptr(d_pos, "float32", 4 * self.n), _dptr(d_col, "float32", 4 * self.n),
+        n = self._count(pair)
+        self.lib.call("sfmb200_copy_to_vbo_coloured", self._h, pair, _dptr(d_pos, "float32", 4 * n), _dptr(d_col, "float32", 4 * n),
                       C.c_float(scale), mode,
                       C.c_float(z_near), C.c_float(z_far))
 

@@ -19,8 +19,10 @@
  *  - a handle owns one device (the current one at create time), one stream and
  *    a pre-sized arena; no allocation happens in any other call.  Handles are
  *    not thread-safe; different handles are independent.
- *  - a handle processes a BATCH of `pairs` image pairs with the same number of
- *    correspondences; SfM::Image_pair is the pairs == 1 case.
+ *  - a handle processes a BATCH of `pairs` image pairs with the same capacity
+ *    (max_points correspondences each); SfM::Image_pair is the pairs == 1 case.
+ *    The pairs hold the same number of correspondences n (set_points_*, run_host,
+ *    run_device) or one count per pair (the *_ragged entry points below).
  *  - there is no CPU fallback: every compute entry point needs a CUDA device.
  */
 #ifndef SFMB200_H
@@ -115,6 +117,32 @@ int sfmb200_set_points_xy(sfmb200_t* h, const float* d_px, int n);
 int sfmb200_set_points_xy_host(sfmb200_t* h, const float* h_px, int n);
 /* already normalised camera coordinates (x1, y1, x2, y2), device [pairs][n][4]. */
 int sfmb200_set_points_normalised(sfmb200_t* h, const float* d_x, int n);
+
+/* ---- batches with a different number of correspondences per pair ----
+ * d_px / h_px: PACKED pixel rows (u1, v1, u2, v2), [offsets[pairs]][4]; pair b owns rows [offsets[b], offsets[b+1]).
+ * h_offsets: HOST int32 [pairs + 1], offsets[0] == 0, every count offsets[b+1] - offsets[b] in [8, max_points].
+ * Contract: pair b of a ragged batch gives the same bits as a one-pair handle holding only pair b's rows
+ * (n = count_b) with the batch's per-pair seed, seed + 0x632BE59BD9B4E019 * b (mod 2^64): inlier counts, best index
+ * and count, E, the four poses and the pose index, the points of its count_b rows and the inlier mask.
+ * Mode: a handle whose last ingest was *_ragged is in per-pair-count mode whatever the counts are; any uniform ingest
+ * (set_points_*, run_device, run_host) returns it to uniform mode.  In per-pair-count mode:
+ *  - estimate_e / _slice / _adaptive, pose_candidates, choose_pose, triangulate, both score metrics, every scoring
+ *    variant and every getter accept the points; the adaptive bound uses w = count / count_b;
+ *  - caller-supplied sample rows keep the [pairs][H_total][8] layout; a row with an index >= count_b is degenerate
+ *    (E = 0, count 0); the disjoint sampler (option 10 = 1) needs 8 * H_total <= the smallest count;
+ *  - per-pair getters (get_points*, get_X, get_inlier_mask, copy_to_vbo*) return count_b entries for pair b;
+ *    device_views keeps point_stride, and rows at or beyond count_b are unspecified there;
+ *  - refine_e, bundle_adjust, chain_views, bundle_adjust_global, find_homography, estimate_e_mg and adopt_best return
+ *    SFMB200_ERR_STATE; the fused small path (option 7) is never taken.
+ * Every argument is checked before anything is enqueued; a refused call leaves the handle as it was.
+ * run_host_ragged: host buffers as run_host; h_points is packed like the input: pair b's [4][count_b] block starts at
+ * float 4 * offsets[b].  E, P, pose index and inliers are [pairs] arrays as in run_host. */
+int sfmb200_set_points_xy_ragged(sfmb200_t* h, const float* d_px, const int32_t* h_offsets);
+int sfmb200_run_device_ragged(sfmb200_t* h, const float* d_px, const int32_t* h_offsets, int H, uint64_t seed, float thr);
+int sfmb200_run_host_ragged(sfmb200_t* h, const float* h_px, const int32_t* h_offsets, int H, uint64_t seed, float thr,
+                            float* h_E, float* h_P, int32_t* h_pose_index, int32_t* h_inliers, float* h_points);
+/* correspondences per pair of the current points (uniform mode: n for every pair) */
+int sfmb200_get_point_counts(sfmb200_t* h, int32_t* h_counts /* [pairs] */);
 
 /* ---- RANSAC: Image_pair::estimateE (SfM/sfm.cu:94-153) + calculateInliers (155-236) ----
  * H hypotheses per pair.  d_idx: device int32 [pairs][H_total][8] sample rows

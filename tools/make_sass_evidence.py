@@ -43,8 +43,8 @@ def longest_loop(lines):
             if best is None or fp > best[0]:
                 best = (fp, body)
     return best[1] if best else []
-targets = [("score", "score_kernelILi8ELb1ELi256ELi1ELi0E", "score_kernel<8, true, 256, 1, 0>: Sampson scoring, packed FFMA2, TMA-staged points (the config-2 / 3 / 4 kernel)"),
-           ("triangulate", "triangulate_kernelILi2ELb0E", "triangulate_kernel<2, false>: two points per thread in packed f32x2"),
+targets = [("score", "score_kernelILi8ELb1ELi256ELi1ELi0ELb0E", "score_kernel<8, true, 256, 1, 0>: Sampson scoring, packed FFMA2, TMA-staged points (the config-2 / 3 / 4 kernel)"),
+           ("triangulate", "triangulate_kernelILi2ELb0ELb0E", "triangulate_kernel<2, false>: two points per thread in packed f32x2"),
            ("hypgen", "hypgen_kernelILi128ELi4ELi0ELi1E", "hypgen_kernel<128, 4, 0, 1>: 8x8 Cholesky projector hypothesis solver"),
            ("small", "small_path_kernel", "small_path_kernel: fused single-launch path, one thread-block cluster per pair")]
 for tag, key, title in targets:
