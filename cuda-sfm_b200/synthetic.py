@@ -124,6 +124,60 @@ def synthetic_sequence(views: int, n: int, outlier_frac: float = 0.2, noise_px: 
     return {"px_views": px, "px_pairs": pairs, "G": G, "X": X, "is_outlier": is_out, "baselines": baselines}
 
 
+def synthetic_orbit(views: int, n: int, noise_px: float = 0.5, seed: int = 2468, radius: float = 6.0,
+                    step_deg=(0.8, 2.0), window=(2, 10), dropout: float = 0.1):
+    """Long N-view sequence (up to a full turn) for the chaining and global-adjustment stages: camera k sits on a circle of
+    the given radius about the scene centre (0, 0, radius), turned by a random step in step_deg degrees per view about the
+    vertical axis and looking at the centre, so baselines (and the relative scales of consecutive pairs) differ.  Camera 0
+    = [I|0].  Each track is seen by a window of consecutive views whose length is drawn from window (inclusive) and which
+    the ends of the sequence may cut short; each view strictly inside the window drops it with probability dropout.  A view that does not see a track holds a uniform pixel
+    for it, one per view: pair k-1's second image and pair k's first image carry the same pixel.
+
+    Returns dict: px_views (views, n, 2) float32, px_pairs (views-1, n, 4) float32 = (view b, view b+1), G (views, 4, 4)
+    world(camera 0)->camera k, X (n, 3), visible (views, n) bool, baselines (views-1,)."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    f, cx, cy = F_REF, W_REF / 2.0, H_REF / 2.0
+    theta = np.concatenate([[0.0], np.cumsum(np.deg2rad(rng.uniform(step_deg[0], step_deg[1], views - 1)))])
+    C = np.array([0.0, 0.0, radius])
+    G = np.tile(np.eye(4), (views, 1, 1))
+    for k, th in enumerate(theta):
+        Rc = _rot([0.0, 1.0, 0.0], np.rad2deg(th))                 # camera -> world; optical axis towards the centre
+        G[k, :3, :3] = Rc.T
+        G[k, :3, 3] = -Rc.T @ (C - radius * Rc[:, 2])
+    baselines = np.linalg.norm(np.diff([-G[k, :3, :3].T @ G[k, :3, 3] for k in range(views)], axis=0), axis=1)
+    lo, hi = window[0], min(window[1], views)
+    length = rng.integers(lo, hi + 1, n)
+    start = (rng.random(n) * (views + length - 1)).astype(int) - (length - 1)     # windows cut by the ends: even coverage
+    k_ = np.arange(views)[:, None]
+    in_window = (k_ >= start) & (k_ < start + length)
+    visible = in_window & ~((k_ > start) & (k_ < start + length - 1) & (rng.random((views, n)) < dropout))
+    X = np.empty((n, 3))
+    todo = np.arange(n)
+    while len(todo):                                               # a point must project into every view of its window
+        P = C + np.stack([rng.uniform(-1, 1, len(todo)), rng.uniform(-0.6, 0.6, len(todo)), rng.uniform(-1, 1, len(todo))], 1)
+        ok = np.ones(len(todo), bool)
+        for k in range(views):
+            w = in_window[k, todo]
+            if not w.any():
+                continue
+            Y = P[w] @ G[k, :3, :3].T + G[k, :3, 3]
+            u, v = f * Y[:, 0] / Y[:, 2] + cx, f * Y[:, 1] / Y[:, 2] + cy
+            ok[np.flatnonzero(w)[~((Y[:, 2] > 0) & (u >= 0) & (u < W_REF) & (v >= 0) & (v < H_REF))]] = False
+        X[todo[ok]] = P[ok]
+        todo = todo[~ok]
+    px = np.empty((views, n, 2))
+    for k in range(views):
+        Y = X @ G[k, :3, :3].T + G[k, :3, 3]
+        px[k, :, 0], px[k, :, 1] = f * Y[:, 0] / Y[:, 2] + cx, f * Y[:, 1] / Y[:, 2] + cy
+    px += rng.normal(0.0, noise_px, px.shape)
+    hidden = ~visible
+    px[hidden, 0] = rng.uniform(0, W_REF, int(hidden.sum()))
+    px[hidden, 1] = rng.uniform(0, H_REF, int(hidden.sum()))
+    px = px.astype(np.float32)
+    pairs = np.concatenate([px[:-1], px[1:]], axis=2)
+    return {"px_views": px, "px_pairs": pairs, "G": G, "X": X, "visible": visible, "baselines": baselines}
+
+
 def planar_pair(n: int, outlier_frac: float = 0.3, noise_px: float = 0.5, seed: int = 7):
     """Correspondences of a planar scene (points on a slanted plane seen by the same two
     cameras as synthetic_pair): image 2 = H(image 1) + noise, plus uniform outliers.

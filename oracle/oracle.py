@@ -49,6 +49,7 @@ reference_K = _synthetic.reference_K
 synthetic_pair = _synthetic.synthetic_pair
 planar_pair = _synthetic.planar_pair
 synthetic_sequence = _synthetic.synthetic_sequence
+synthetic_orbit = _synthetic.synthetic_orbit
 
 
 def normalise_points(px: np.ndarray, Kinv: np.ndarray) -> np.ndarray:
@@ -679,7 +680,7 @@ def bundle_adjust(x: np.ndarray, M: np.ndarray, X: np.ndarray, active: np.ndarra
     Mo[:3, :3], Mo[:3, 3] = R, t * sc
     Xo = triangulate(x, Mo)     # whole cloud under the refined camera; adjusted points for the active set
     Xo[:3, act] = (Xc * sc).T
-    return dict(M=Mo, X=Xo, cost0=cost0, cost=cost, accepted=accepted, n_active=len(act))
+    return dict(M=Mo, X=Xo, cost0=cost0, cost=cost, accepted=accepted, n_active=len(act), gauge_scale=sc)
 
 
 def essential_from_pose(M: np.ndarray) -> np.ndarray:
@@ -880,6 +881,86 @@ def bundle_adjust_global(uv, obs, G, X, iterations: int = 30, lam0: float = 1e-3
             Gn[k][:3, 3] = G[k][:3, 3] + dt
         Xn = X.copy()
         Xn[:, act] += d[ncam:].reshape(-1, 3).T
+        cn = gba_cost(uv, obs, Gn, Xn)
+        if np.isfinite(cn) and cn < cost:
+            G, X, cost, accepted = Gn, Xn, cn, accepted + 1
+            lam = max(lam / 3, 1e-9)
+        else:
+            lam = min(4 * lam, 1e6)
+    sc = t1 / np.linalg.norm(G[1][:3, 3]) if V > 1 else 1.0
+    G[:, :3, 3] *= sc
+    X[:, act] *= sc
+    return G, X, {"cost_entry": cost0, "cost": cost, "accepted": accepted, "lambda": lam, "gauge_scale": sc}
+
+
+def bundle_adjust_global_schur(uv, obs, G, X, iterations: int = 30, lam0: float = 1e-3):
+    """bundle_adjust_global restated the way chain.cu computes the step, for sequences and track counts where the dense
+    Jacobian is too large: per view the residuals and Jacobians of all its observations at once, the damped 3x3 point
+    blocks inverted as a batch, the reduced camera system S dc = -rhs of 6 (V-1) unknowns assembled from them and solved
+    densely, then the back-substitution dX_i = -V_i*^-1 (g_p,i + sum_k W_ki^T dc_k).  Same damping (diagonal x (1 + lambda)),
+    accept rule, lambda schedule and gauge as the dense version; same returns."""
+    V, n = obs.shape
+    G = np.array(G, float).copy()
+    X = np.array(X, float)[:3].copy()
+    act = np.flatnonzero(obs.any(0))
+    P, K = len(act), V - 1
+    ob = obs[:, act]
+    t1 = np.linalg.norm(G[1][:3, 3]) if V > 1 else 1.0
+    lam = lam0
+    cost = gba_cost(uv, obs, G, X)
+    cost0, accepted = cost, 0
+    for _ in range(iterations):
+        Vp = np.zeros((P, 3, 3))
+        gp = np.zeros((P, 3))
+        W = np.zeros((P, K, 6, 3))                          # W_ki = Jc^T Jp, zero where view k does not see track i
+        U = np.zeros((K, 6, 6))
+        gc = np.zeros((K, 6))
+        Xa = X[:, act].T
+        for k in range(V):
+            j = np.flatnonzero(ob[k])
+            R, t = G[k][:3, :3], G[k][:3, 3]
+            Q = Xa[j] @ R.T
+            Y = Q + t
+            iz = 1.0 / Y[:, 2]
+            u, v = Y[:, 0] * iz, Y[:, 1] * iz
+            r = np.stack([u - uv[k][act[j], 0], v - uv[k][act[j], 1]], 1)
+            bp = np.zeros((len(j), 2, 3))
+            bp[:, 0, 0] = iz; bp[:, 0, 2] = -u * iz
+            bp[:, 1, 1] = iz; bp[:, 1, 2] = -v * iz
+            Jp = bp @ R
+            Vp[j] += Jp.transpose(0, 2, 1) @ Jp
+            gp[j] += (Jp.transpose(0, 2, 1) @ r[:, :, None])[:, :, 0]
+            if k == 0:
+                continue
+            N = np.zeros((len(j), 3, 3))                      # -[Q]x
+            N[:, 0, 1] = Q[:, 2]; N[:, 0, 2] = -Q[:, 1]
+            N[:, 1, 0] = -Q[:, 2]; N[:, 1, 2] = Q[:, 0]
+            N[:, 2, 0] = Q[:, 1]; N[:, 2, 1] = -Q[:, 0]
+            Jc = np.concatenate([bp @ N, bp], axis=2)
+            U[k - 1] = np.einsum("mra,mrb->ab", Jc, Jc)
+            gc[k - 1] = np.einsum("mra,mr->a", Jc, r)
+            W[j, k - 1] = Jc.transpose(0, 2, 1) @ Jp
+        Vp[:, np.arange(3), np.arange(3)] *= 1.0 + lam
+        U[:, np.arange(6), np.arange(6)] *= 1.0 + lam
+        Vinv = np.linalg.inv(Vp)
+        T = np.einsum("pkac,pcd->pkad", W, Vinv)            # W_ki V_i*^-1
+        S = -np.einsum("pkad,plbd->kalb", T, W).reshape(6 * K, 6 * K)
+        for k in range(K):
+            S[6 * k: 6 * k + 6, 6 * k: 6 * k + 6] += U[k]
+        rhs = (gc - np.einsum("pkad,pd->ka", T, gp)).reshape(-1)
+        try:
+            dc = np.linalg.solve(S, -rhs)
+        except np.linalg.LinAlgError:
+            lam = min(4 * lam, 1e6)
+            continue
+        dX = -np.einsum("pcd,pd->pc", Vinv, gp + np.einsum("pkac,ka->pc", W, dc.reshape(K, 6)))
+        Gn = G.copy()
+        for k in range(1, V):
+            w, dt = dc[6 * (k - 1): 6 * (k - 1) + 3], dc[6 * (k - 1) + 3: 6 * (k - 1) + 6]
+            Gn[k][:3, :3] = _rodrigues(w) @ G[k][:3, :3]
+            Gn[k][:3, 3] = G[k][:3, 3] + dt
+        Xn = X.copy()
+        Xn[:, act] += dX.T
         cn = gba_cost(uv, obs, Gn, Xn)
         if np.isfinite(cn) and cn < cost:
             G, X, cost, accepted = Gn, Xn, cn, accepted + 1

@@ -350,3 +350,79 @@ def test_global_bundle_adjustment_restatement_converges(O):
     err0 = np.median(np.linalg.norm(X0 - Xt, axis=0) / np.linalg.norm(Xt, axis=0))
     err1 = np.median(np.linalg.norm(X / s_true - Xt, axis=0) / np.linalg.norm(Xt, axis=0))
     assert err1 < err0
+
+
+def _digest(d):
+    import hashlib
+
+    m = hashlib.sha256()
+    for k in sorted(d):
+        m.update(k.encode())
+        m.update(np.ascontiguousarray(d[k]).tobytes())
+    return m.hexdigest()
+
+
+def test_synthetic_sequence_default_output_is_pinned(O):
+    """The chaining and bundle-adjustment tests were tuned on these exact sequences: the generator's default output must not
+    drift when the generators beside it change."""
+    assert _digest(O.synthetic_sequence(4, 500, seed=4321)) == "b7aa80f72bf13d7929d58f8e81c8f484c40999cc01796edacc89917e83d8467b"
+    assert _digest(O.synthetic_sequence(4, 500, seed=99)) == "4fea257fda6fbdfbaa4bef179693f4c7d514c27852aaa08ee5fde3660be6adbd"
+    assert _digest(O.synthetic_sequence(3, 300)) == "fdff9d526563b6568402d384df6b0e4f076debc0dfc9be7a9f1aee5dcaedb77f"
+
+
+def test_synthetic_orbit_visibility_and_geometry(O):
+    views, n = 65, 6000
+    sc = O.synthetic_orbit(views, n)
+    G, vis, px = sc["G"], sc["visible"], sc["px_views"].astype(np.float64)
+    assert np.allclose(G[0], np.eye(4)) and sc["px_pairs"].shape == (views - 1, n, 4)
+    # one pixel per view: pair k-1's second image is pair k's first image
+    assert np.array_equal(sc["px_pairs"][:-1, :, 2:], sc["px_pairs"][1:, :, :2])
+    assert np.array_equal(sc["px_pairs"][0, :, :2], sc["px_views"][0]) and np.array_equal(sc["px_pairs"][-1, :, 2:], sc["px_views"][-1])
+    # visible observations are the projections of X up to the pixel noise, all inside the image
+    f, cx, cy = O.F_REF, O.W_REF / 2, O.H_REF / 2
+    for k in (0, 31, views - 1):
+        Y = sc["X"] @ G[k][:3, :3].T + G[k][:3, 3]
+        proj = np.stack([f * Y[:, 0] / Y[:, 2] + cx, f * Y[:, 1] / Y[:, 2] + cy], 1)
+        m = vis[k]
+        assert np.all(Y[m, 2] > 0) and np.abs(proj[m] - px[k][m]).max() < 4.0
+        assert np.all((px[k] >= 0).all(1) & (px[k][:, 0] < O.W_REF) & (px[k][:, 1] < O.H_REF))
+    # windows of 2..10 views with gaps inside, even coverage of the pairs, baselines of different lengths
+    seen = vis.sum(0)
+    assert seen.max() <= 10 and (seen >= 2).mean() > 0.9
+    first, last = vis.argmax(0), views - 1 - vis[::-1].argmax(0)
+    assert np.sum(last - first + 1 > seen) > 0.1 * n                 # dropouts leave gaps
+    live = (vis[:-1] & vis[1:]).sum(1)
+    assert live.min() > 0.6 * live.mean()
+    assert sc["baselines"].max() / sc["baselines"].min() > 1.8
+    # the same arguments give the same bits
+    assert _digest(O.synthetic_orbit(9, 300, seed=5)) == _digest(O.synthetic_orbit(9, 300, seed=5))
+
+
+@pytest.mark.parametrize("views", [2, 3, 5])
+@pytest.mark.parametrize("iterations", [1, 10])
+def test_global_ba_schur_restatement_equals_dense(O, views, iterations):
+    """oracle.bundle_adjust_global_schur (per-view vectorised, points eliminated) takes the same steps as the dense
+    restatement oracle.bundle_adjust_global, on tracks that only part of the views see."""
+    K, Kinv = O.reference_K()
+    n = 120
+    sc = O.synthetic_orbit(views, n, noise_px=0.5, seed=30 + views, window=(2, 4), dropout=0.3)
+    xs = [O.normalise_points(sc["px_pairs"][b], Kinv).astype(np.float64) for b in range(views - 1)]
+    valids = [sc["visible"][b] & sc["visible"][b + 1] for b in range(views - 1)]
+    uv, obs = O.gba_observations(xs, valids)
+    if views > 2:
+        assert (~obs).any() and obs.any(0).sum() > 0.5 * n                 # partial visibility
+    rng = np.random.default_rng(views)
+    Gt = sc["G"].copy()
+    G0 = Gt.copy()
+    for k in range(1, views):
+        G0[k][:3, :3] = O._rodrigues(rng.normal(size=3) * 0.003) @ Gt[k][:3, :3]
+        G0[k][:3, 3] += rng.normal(size=3) * 0.01
+    X0 = sc["X"].T * (1 + rng.normal(size=(3, n)) * 0.005)
+    Gd, Xd, sd = O.bundle_adjust_global(uv, obs, G0, X0, iterations=iterations)
+    Gs, Xs, ss = O.bundle_adjust_global_schur(uv, obs, G0, X0, iterations=iterations)
+    assert sd["accepted"] >= 1 and sd["cost"] < sd["cost_entry"]
+    assert sd["accepted"] == ss["accepted"] and sd["lambda"] == ss["lambda"]
+    for k in ("cost_entry", "cost", "gauge_scale"):
+        assert abs(sd[k] - ss[k]) <= 1e-9 * abs(sd[k]), k
+    assert np.abs(Gd - Gs).max() < 1e-9
+    assert np.abs(Xd - Xs).max() < 1e-9 * np.abs(Xd).max()
